@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU implementation (oracle port)
+    python bench.py --steps K --dump-outputs DIR             # also write what the last timed step computed, as .npy
 
 Workload (BASELINE.json configs[1]; SURVEY.md 8d "C2"): F=10 features (CAN ID, DLC, 8 data bytes), K=5
 classes, Z=128, fp32, batch 4096 rows PER GPU (weak scaling: global batch 4096*N).  One bench "step" is
@@ -256,6 +257,23 @@ def run_reference(args):
     print(json.dumps(line), flush=True)
 
 
+def dump_outputs(out_dir, eng, loss):
+    """What the timed label visits hand back to a caller, as float32 .npy files (about 1 MB in all): `losses.npy`, the
+    13 x 4 losses of the last visit, and `<network>.<state_dict key>.npy` for every tensor of the four networks after it.
+    The inputs depend only on the command-line arguments.  Weight and LayerNorm-affine gradients are summed exactly (fixed
+    point, gemm_dw_kernel / ln_bwd_kernel), so the order the GPU adds them in cannot change them; BatchNorm statistics and
+    loss sums still use double-precision atomics, whose order can move the last bit of a double before it is rounded to
+    float32.  Measured on one B200 (1000 W limit): two runs with the same arguments wrote bit-identical files at --steps 1,
+    50 and 100."""
+    import numpy as np
+    from cvae_gan_b200._lib import NET_NAMES
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "losses.npy"), loss.cpu().numpy())
+    for net, name in enumerate(NET_NAMES):
+        for key, t in eng.export_state(net).items():
+            np.save(os.path.join(out_dir, f"{name}.{key}.npy"), t.cpu().numpy())
+
+
 def _finish(eng, world):
     """Leave the process without running communicator destructors: with several ranks, tearing down the library's NCCL
     communicator and torch's process group in arbitrary order has been seen to block for minutes after the result line
@@ -407,6 +425,8 @@ def run_ours(args):
     ms = timed(visit_resident, args.steps, warm)
     launches = launches_per_visit * args.steps
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng, loss)     # before the e2e visits below overwrite losses and weights
     ms_e2e = timed(visit_e2e, args.steps, 1)
     value = OPT_STEPS * Bg * args.steps / (ms * 1e-3)
     e2e = OPT_STEPS * Bg * args.steps / (ms_e2e * 1e-3)
@@ -460,7 +480,7 @@ def run_ours(args):
                 with torch.cuda.graph(g):
                     eng.visit(label, Bg, class_rows=tabs[label], loops=LOOPS, loss_out=loss)
                 pg[label] = g
-            k_prog = max(5, min(args.steps, 40))
+            k_prog = args.steps
             ms_p = timed(lambda lab: pg[lab].replay(), k_prog, 3)
             train_program = {
                 "ms_per_step": ms_p / k_prog, "value": OPT_STEPS * Bg * k_prog / (ms_p * 1e-3), "unit": "samples/s", "steps": k_prog,
@@ -480,7 +500,7 @@ def run_ours(args):
     train_wide = None
     if world == 1 and not args.no_wide:
         try:
-            train_wide = run_wide_leg(dev, tabs, timed, pk, max(5, min(args.steps, 20)))
+            train_wide = run_wide_leg(dev, tabs, timed, pk, args.steps)
         except Exception as ex:
             train_wide = {"error": str(ex)[:300]}
 
@@ -862,7 +882,13 @@ def main():
     ap.add_argument("--no-wide", action="store_true", help="skip the widened-model leg (BASELINE.json configs[4], fp32, 1 GPU)")
     ap.add_argument("--only-filter", action="store_true", help="dev aid: run only the generation + filter leg")
     ap.add_argument("--quick", action="store_true", help="profiling aid (ncu): resident loop only, no e2e/cpu legs; NOT a bench number")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the losses of the last timed label visit "
+                                                          "and the four networks' state after it to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.quick or args.only_filter):
+        ap.error("--dump-outputs writes the outputs of the training visits timed by --impl ours (not --quick / --only-filter)")
     if args.impl == "reference":
         run_reference(args)
     else:

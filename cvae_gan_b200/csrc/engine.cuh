@@ -12,6 +12,8 @@ namespace cvg {
 constexpr int HOIST_MAX = 16;  // generator passes one hoisted forward can hold (d_loop + c_loop of a visit)
 constexpr int STAT_C = 1024;   // max features of a BatchNorm layer (stats slots are [2][STAT_C])
 
+constexpr int DET_MAX_PASS = 4;   // passes per launch the deterministic-reduction slots are sized for
+
 // feature-major workspace (all float matrices are [features][ld], two pass slots where noted)
 struct Workspace {
   int ld = 0;          // rows rounded up to 64
@@ -78,6 +80,13 @@ struct Workspace {
   // step-program kernel (mega.cuh): weight-gradient partial slots, grid-barrier counter, materialised z_enc slot
   float* dw_scratch = nullptr;
   long long dw_scratch_floats = 0;
+  // stand-alone kernels' deterministic reductions (gemm_dw_kernel, ln_bwd_kernel): fixed-point accumulators and ticket
+  // counters, one set per stream the engine launches on (0: the caller's, 1 / 2: the side streams), since launches on one
+  // stream never overlap
+  unsigned long long* det_acc[3] = {};
+  unsigned* det_cnt[3] = {};
+  long long det_acc_n = 0;
+  int det_cnt_n = 0;
   unsigned int* mk_bar = nullptr;
   float* z_eps = nullptr;          // [Z][ld] reparameterisation noise of the E+G step when the program kernel runs it
   float* mk_wprep = nullptr;       // hi / lo pre-split weight chunks of every layer, both GEMM orientations

@@ -645,8 +645,18 @@ __global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_mn_kernel(const GemmArgs
 constexpr int DW_MC = 32;          // batch rows per staged chunk
 constexpr int DW_LDS = DW_MC + 4;  // padded row (conflict-free 128-bit reads across rows)
 
+// Deterministic split-batch reduction: each CTA adds its partial tile to `acc` ([tile][pass] slots of DW_PART int64) in
+// fixed point (DET_FIX_SCALE), where addition is exact and so independent of the order the CTAs finish in; the last CTA of
+// the tile (ticket on `tile_cnt`) converts the sums, adds them to the gradients and clears the slot and the counter.
+constexpr int DW_PART = 64 * 64 + 64;   // dW tile + bias sums
+constexpr double DET_FIX_SCALE = 1099511627776.0;   // 2^40: resolution 9.1e-13, range +-8.4e6
+__device__ __forceinline__ unsigned long long det_fix(float v) {
+  return (unsigned long long)__double2ll_rn((double)v * DET_FIX_SCALE);
+}
+__device__ __forceinline__ float det_unfix(unsigned long long v) { return (float)((double)(long long)v / DET_FIX_SCALE); }
+
 template <int PK, int QK>
-__global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_dw_kernel(const DwArgs g, int nsplit) {
+__global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_dw_kernel(const DwArgs g, int nsplit, unsigned long long* acc64, unsigned* tile_cnt) {
   extern __shared__ __align__(16) float dyn_smem[];
   float* Ps = dyn_smem;                            // [2][64][DW_LDS]
   float* Qs = Ps + 2 * 64 * DW_LDS;                // [2][64][DW_LDS]
@@ -674,15 +684,8 @@ __global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_dw_kernel(const DwArgs g
   operand_consts<QK>(g.q, pass, g.Bg, g.bn_eps, cs_q, poll_q);
   // BatchNorm affine gradients are exactly the backward batch sums (appendix A.2): dbeta = sum dy,
   // dgamma = sum dy*xhat.  One CTA per pass adds them to the gradient buffer.
-  if (g.add_affine && g.dgamma && blockIdx.x == 0 && blockIdx.y == 0 && split == 0) {
-    const double* bs = g.p.bn.bstats + (long long)pass * g.p.bn.sb;
-    for (int c = tid; c < g.p.bn.C; c += GEMM_THREADS) {
-      atomicAdd(g.dbeta + c, (float)bs[c]);
-      atomicAdd(g.dgamma + c, (float)bs[g.p.bn.C + c]);
-    }
-  }
+  // (added by the last CTA of tile (0, 0), pass by pass)
   __syncthreads();
-  if (mbeg >= mend) return;
 
   const int l_row = tid >> 3, l_m = (tid & 7) * 4;   // two rows per thread: l_row, l_row + 32
   const int tk = tid & 15, tn = tid >> 4;            // thread computes rows tn+16i (n) x tk+16j (k)
@@ -740,10 +743,12 @@ __global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_dw_kernel(const DwArgs g
     }
   };
 
-  const int nchunks = (mend - mbeg + DW_MC - 1) / DW_MC;
+  const int nchunks = mbeg < mend ? (mend - mbeg + DW_MC - 1) / DW_MC : 0;
   Regs rr;
-  gload(mbeg, rr);
-  sstore(0, mbeg, rr);
+  if (nchunks > 0) {
+    gload(mbeg, rr);
+    sstore(0, mbeg, rr);
+  }
   __syncthreads();
   for (int c = 0; c < nchunks; ++c) {
     const int cur = c & 1;
@@ -753,21 +758,53 @@ __global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_dw_kernel(const DwArgs g
     __syncthreads();
   }
 
-  float* dW = g.dW + (long long)pass * g.sdW;
+  const int tile = blockIdx.y * gridDim.x + blockIdx.x;
+  unsigned long long* tacc = acc64 + (size_t)tile * g.npass * DW_PART;
+  {
+    unsigned long long* mine = tacc + (size_t)pass * DW_PART;
 #pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int n = n0 + tn + 16 * i;
-    if (n >= g.N) continue;
+    for (int i = 0; i < 4; ++i) {
+      const int n = n0 + tn + 16 * i;
+      if (n >= g.N) continue;
 #pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const int k = k0 + tk + 16 * j;
-      if (k < g.K) atomicAdd(dW + (size_t)n * g.ldw + g.wcol0 + k, acc[i][j]);
-    }
-    if (do_bias) {
-      if (g.db) atomicAdd(g.db + n, bsum[i]);
-      if (g.label_col >= 0) atomicAdd(dW + (size_t)n * g.ldw + g.label_col, bsum[i]);
+      for (int j = 0; j < 4; ++j)
+        if (k0 + tk + 16 * j < g.K) atomicAdd(mine + (tn + 16 * i) * 64 + tk + 16 * j, det_fix(acc[i][j]));
+      if (do_bias) atomicAdd(mine + 64 * 64 + tn + 16 * i, det_fix(bsum[i]));
     }
   }
+  __threadfence();
+  __syncthreads();
+  __shared__ unsigned s_last;
+  if (tid == 0) s_last = atomicAdd(tile_cnt + tile, 1u) == gridDim.z - 1 ? 1u : 0u;
+  __syncthreads();
+  if (!s_last) return;
+  __threadfence();
+  for (int ps = 0; ps < g.npass; ++ps) {
+    if (g.add_affine && g.dgamma && tile == 0) {
+      const double* bs = g.p.bn.bstats + (long long)ps * g.p.bn.sb;
+      for (int c = tid; c < g.p.bn.C; c += GEMM_THREADS) {
+        atomicAdd(g.dbeta + c, (float)__ldcg(bs + c));               // written by this pass's write-back CTA
+        atomicAdd(g.dgamma + c, (float)__ldcg(bs + g.p.bn.C + c));
+      }
+    }
+    unsigned long long* pa = tacc + (size_t)ps * DW_PART;
+    float* dW = g.dW + (long long)ps * g.sdW;
+    const bool bias = (g.db != nullptr || g.label_col >= 0) && blockIdx.x == 0;
+    for (int el = tid; el < DW_PART; el += GEMM_THREADS) {
+      const bool is_b = el >= 64 * 64;
+      const int n = n0 + (is_b ? el - 64 * 64 : el >> 6), k = k0 + (el & 63);
+      if (n >= g.N || (is_b ? !bias : k >= g.K)) continue;
+      const float sum = det_unfix(__ldcg(pa + el));
+      pa[el] = 0ull;
+      if (!is_b) {
+        atomicAdd(dW + (size_t)n * g.ldw + g.wcol0 + k, sum);
+      } else {
+        if (g.db) atomicAdd(g.db + n, sum);
+        if (g.label_col >= 0) atomicAdd(dW + (size_t)n * g.ldw + g.label_col, sum);
+      }
+    }
+  }
+  if (tid == 0) tile_cnt[tile] = 0u;
 }
 
 inline size_t gemm_mn_smem(const GemmArgs& g) {
@@ -808,14 +845,16 @@ inline cudaError_t dispatch_mn(bool wt, const GemmArgs& g, dim3 grid, size_t sme
 }
 
 template <int PK, int QK>
-inline cudaError_t launch_dw_inst(const DwArgs& g, int nsplit, dim3 grid, size_t smem, cudaStream_t st) {
-  gemm_dw_kernel<PK, QK><<<grid, GEMM_THREADS, smem, st>>>(g, nsplit);
+inline cudaError_t launch_dw_inst(const DwArgs& g, int nsplit, unsigned long long* acc, unsigned* cnt, dim3 grid,
+                                  size_t smem, cudaStream_t st) {
+  gemm_dw_kernel<PK, QK><<<grid, GEMM_THREADS, smem, st>>>(g, nsplit, acc, cnt);
   return cudaGetLastError();
 }
 
-inline cudaError_t dispatch_dw(const DwArgs& g, int nsplit, dim3 grid, size_t smem, cudaStream_t st) {
+inline cudaError_t dispatch_dw(const DwArgs& g, int nsplit, unsigned long long* acc, unsigned* cnt, dim3 grid,
+                               size_t smem, cudaStream_t st) {
 #define CVG_DW(P, Q) \
-  if (g.p.kind == P && g.q.kind == Q) return launch_dw_inst<P, Q>(g, nsplit, grid, smem, st);
+  if (g.p.kind == P && g.q.kind == Q) return launch_dw_inst<P, Q>(g, nsplit, acc, cnt, grid, smem, st);
   CVG_DW(OP_PLAIN, OP_PLAIN)
   CVG_DW(OP_CONST, OP_PLAIN)
   CVG_DW(OP_PLAIN, OP_BN_ACT)

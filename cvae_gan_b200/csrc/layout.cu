@@ -250,6 +250,21 @@ static size_t carve(const Engine& e, Workspace& w, void* base) {
   }
   w.dw_scratch = c.take<float>((size_t)w.dw_scratch_floats);
   {
+    int tiles = 1, cmax = 1;
+    for (int net = 0; net < 4; ++net)
+      for (int i = 0; i < e.lay[net].nlin; ++i) {
+        const LinearP& p = e.lay[net].lin[i];
+        tiles = std::max(tiles, ((p.in + 63) / 64) * ((p.out + 63) / 64));
+        cmax = std::max(cmax, std::max(p.in, p.out));
+      }
+    w.det_acc_n = std::max((long long)tiles * DET_MAX_PASS * DW_PART, 2LL * cmax);
+    w.det_cnt_n = tiles;
+    for (int i = 0; i < 3; ++i) {
+      w.det_acc[i] = c.take<unsigned long long>((size_t)w.det_acc_n);
+      w.det_cnt[i] = c.take<unsigned>((size_t)w.det_cnt_n);
+    }
+  }
+  {
     // pre-split weight chunks (128 rows x 32 k, hi + lo = 8192 floats): both orientations of every Linear; the heads and
     // first layers are prepped with a narrower contraction, never a wider one
     long long chunks = 0;

@@ -133,8 +133,10 @@ struct LnBwdArgs {
   float* dg; float* db;                // null -> skipped
 };
 
+// The affine gradients are summed in fixed point in `acc` ([2C] int64, det_fix: exact, so independent of the block order);
+// the last block (ticket on `cnt`) converts them, adds them to dg / db and clears `acc` and `cnt` (like gemm_dw_kernel).
 template <int MAXF>
-__global__ void __launch_bounds__(256) ln_bwd_kernel(const LnBwdArgs g) {
+__global__ void __launch_bounds__(256) ln_bwd_kernel(const LnBwdArgs g, unsigned long long* acc, unsigned* cnt) {
   __shared__ float red1[8][LN_ROWS], red2[8][LN_ROWS];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
   const int m = blockIdx.x * LN_ROWS + lane;
@@ -176,11 +178,25 @@ __global__ void __launch_bounds__(256) ln_bwd_kernel(const LnBwdArgs g) {
     if (g.dg) {
       const float a = warp_sum(d[i] * xh[i]), b = warp_sum(d[i]);
       if (lane == 0) {
-        atomicAdd(g.dg + c, a);
-        atomicAdd(g.db + c, b);
+        atomicAdd(acc + c, det_fix(a));
+        atomicAdd(acc + g.C + c, det_fix(b));
       }
     }
   }
+  if (!g.dg) return;
+  __threadfence();
+  __syncthreads();
+  __shared__ unsigned s_last;
+  if (threadIdx.x == 0) s_last = atomicAdd(cnt, 1u) == gridDim.x * gridDim.y - 1 ? 1u : 0u;
+  __syncthreads();
+  if (!s_last) return;
+  __threadfence();
+  for (int e = threadIdx.x; e < 2 * g.C; e += blockDim.x) {
+    const float v = det_unfix(__ldcg(acc + e));
+    acc[e] = 0ull;
+    atomicAdd(e < g.C ? g.dg + e : g.db + (e - g.C), v);
+  }
+  if (threadIdx.x == 0) *cnt = 0u;
 }
 
 inline void launch_ln_fwd(const LnArgs& a, cudaStream_t st) {
@@ -188,10 +204,10 @@ inline void launch_ln_fwd(const LnArgs& a, cudaStream_t st) {
   if (a.C <= 8 * LN_MAXF) ln_fwd_kernel<LN_MAXF><<<grid, 256, 0, st>>>(a);
   else ln_fwd_kernel<LN_MAXF_WIDE><<<grid, 256, 0, st>>>(a);
 }
-inline void launch_ln_bwd(const LnBwdArgs& a, cudaStream_t st) {
+inline void launch_ln_bwd(const LnBwdArgs& a, unsigned long long* acc, unsigned* cnt, cudaStream_t st) {
   const dim3 grid((a.M + LN_ROWS - 1) / LN_ROWS, a.npass);
-  if (a.C <= 8 * LN_MAXF) ln_bwd_kernel<LN_MAXF><<<grid, 256, 0, st>>>(a);
-  else ln_bwd_kernel<LN_MAXF_WIDE><<<grid, 256, 0, st>>>(a);
+  if (a.C <= 8 * LN_MAXF) ln_bwd_kernel<LN_MAXF><<<grid, 256, 0, st>>>(a, acc, cnt);
+  else ln_bwd_kernel<LN_MAXF_WIDE><<<grid, 256, 0, st>>>(a, acc, cnt);
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -264,6 +264,9 @@ int launch_mn(Engine& e, bool wt, const GemmArgs& g_in, cudaStream_t st) {
   return 0;
 }
 
+// the deterministic-reduction slot set of the stream a stand-alone kernel is launched on (Workspace::det_acc)
+static int det_slot(const Engine& e, cudaStream_t st) { return st == e.ms.s[0] ? 1 : st == e.ms.s[1] ? 2 : 0; }
+
 int launch_dw(Engine& e, const DwArgs& g0, cudaStream_t st) {
   if (e.mk.recording) return mk_push_dw(e, g0);
   DwArgs g = g0;
@@ -280,8 +283,11 @@ int launch_dw(Engine& e, const DwArgs& g0, cudaStream_t st) {
   if (const NvlDev* ch = take_pending(e, g.p)) g.nvl = ch;
   if (const NvlDev* ch = take_pending(e, g.q)) g.nvl = ch;
   dim3 grid(kt, nt, g.npass * nsplit);
+  if ((long long)kt * nt * g.npass * DW_PART > e.ws.det_acc_n || kt * nt > e.ws.det_cnt_n)
+    CVG_FAIL("internal: weight-gradient launch exceeds the deterministic-reduction slots");
+  const int slot = det_slot(e, st);
   prof_begin(e, 2, 2.0 * g.M * (double)g.N * g.K * g.npass, st);
-  const cudaError_t err = dispatch_dw(g, nsplit, grid, gemm_dw_smem(g), st);
+  const cudaError_t err = dispatch_dw(g, nsplit, e.ws.det_acc[slot], e.ws.det_cnt[slot], grid, gemm_dw_smem(g), st);
   prof_end(e, st);
   if (err != cudaSuccess)
     CVG_FAIL(std::string("gemm_dw launch (p.kind ") + std::to_string(g.p.kind) + ", q.kind " + std::to_string(g.q.kind) +
@@ -854,7 +860,9 @@ static int bwd_classifier(Engine& e, const float* xin, long long sxin, int npass
       if (e.mk.recording) {
         CVG_TRY(mk_push(e, mk::K_LN_BWD, &a, sizeof(a), npass * ((M + 31) / 32)));
       } else {
-        launch_ln_bwd(a, st);
+        const int slot = det_slot(e, st);
+        if (2LL * a.C > e.ws.det_acc_n) CVG_FAIL("internal: LayerNorm backward exceeds the deterministic-reduction slots");
+        launch_ln_bwd(a, e.ws.det_acc[slot], e.ws.det_cnt[slot], st);
         CVG_LAUNCH_CHECK();
       }
     }

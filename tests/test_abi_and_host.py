@@ -62,6 +62,17 @@ def test_lambda_class_schedule_matches_oracle():
         assert lambda_class_at(e, 0.5) == O.lambda_class_schedule(e, 0.5)
 
 
+def _assert_init_equal(got, ref, where):
+    """Everything drawn from the seeded generator must be bit-identical.  Spectral norm's `_u` / `_v` are 15 power-iteration
+    steps (torch.mv) run at construction: the BLAS code path the host CPU selects moves their last bits, so those two
+    vectors are held to 1e-6.  The fixtures match bit for bit where MKL runs its AVX-512 kernels; on the same host,
+    MKL_ENABLE_INSTRUCTIONS=AVX2 (or SSE4_2) moves `_u` / `_v` by up to 2e-7 (7 ulp) and nothing else."""
+    if where[-1].endswith(("._u", "._v")):
+        torch.testing.assert_close(got, ref, rtol=1e-5, atol=1e-6, msg=str(where))
+    else:
+        assert torch.equal(got, ref), where
+
+
 def test_model_mirrors_reproduce_reference_init(golden_dir):
     """Same seed -> same starting parameters as the reference constructor (fixture: reference state_dicts
     right after `set_random_state(); CVAEGAN()`, see oracle/make_golden.py)."""
@@ -80,8 +91,7 @@ def test_model_mirrors_reproduce_reference_init(golden_dir):
         ref_keys = [k.split("/", 2)[2] for k in npz.files if k.startswith(f"init/{name}/")]
         assert list(sd.keys()) == ref_keys
         for k, v in sd.items():
-            ref = torch.from_numpy(npz[f"init/{name}/{k}"])
-            assert torch.equal(v, ref), (name, k)
+            _assert_init_equal(v, torch.from_numpy(npz[f"init/{name}/{k}"]), (name, k))
         assert [k for k, _, _ in O.tensor_table(name, 10, 5, 128)] == ref_keys
 
 
@@ -223,7 +233,7 @@ def test_host_classes_build_networks_in_the_reference_order(golden_dir, cls_name
         ref_keys = [k.split("/", 2)[2] for k in npz.files if k.startswith(f"init/{name}/")]
         assert list(sd.keys()) == ref_keys
         for k, v in sd.items():
-            assert torch.equal(v, torch.from_numpy(npz[f"init/{name}/{k}"])), (cls_name, name, k)
+            _assert_init_equal(v, torch.from_numpy(npz[f"init/{name}/{k}"]), (cls_name, name, k))
     # the extra networks did not advance the generator: the next draw is the one the reference would make
     random.seed(0); np.random.seed(0); torch.manual_seed(0)
     from cvae_gan_b200 import models

@@ -99,7 +99,9 @@ def _worker(rank, world, port, q, trainer="cvae_gan"):
     losses = _run(orc, slice(rank * per, (rank + 1) * per), trainer)
     st = orc.state()
     flat = torch.cat([t.flatten().float() for n in O.NETS for t in st[n].values()])
-    q.put((rank, losses, flat))
+    # a numpy copy, not the tensor: torch.multiprocessing passes tensors by file descriptor, which the parent can only
+    # fetch while this process lives, and it exits right after the barrier below
+    q.put((rank, losses, flat.numpy()))
     dist.barrier()
     dist.destroy_process_group()
 
@@ -117,7 +119,7 @@ def test_dp2_equals_single_process(trainer):
     procs = [ctx.Process(target=_worker, args=(r, 2, port, q, trainer)) for r in range(2)]
     for p in procs:
         p.start()
-    results = [q.get(timeout=300) for _ in range(2)]
+    results = [(rank, losses, torch.from_numpy(flat)) for rank, losses, flat in (q.get(timeout=300) for _ in range(2))]
     for p in procs:
         p.join(timeout=60)
         assert p.exitcode == 0
