@@ -500,6 +500,7 @@ int cvg_debug_set(CvgHandle* h, const char* key, int value) {
   else if (k == "mk_coop") e.mk.coop = value != 0;
   else if (k == "hoist") e.hoist = value != 0;
   else if (k == "streams") e.ms.on = value != 0;
+  else if (k == "chain") e.chain = value != 0;      // 0: the D / C steps run the layer kernels (the chains' reference)
   else if (k == "fuse_stats") e.nvl.fuse = value != 0;
   else CVG_FAIL("cvg_debug_set: unknown key");
   return 0;

@@ -178,6 +178,7 @@ struct Engine {
   bool in_visit = false;            // steps emitted by visit(): their gradient reduction + Adam may run beside the next step
   unsigned long long step_dcounter = 0;   // visit(): Philox counter values the step being emitted uses (advanced at its end)
   int hoist = 1;                    // CVG_HOIST=0: every step runs its own generator forward
+  bool chain = true;                // D / C steps run the critic / classifier as fused row-tile chains (chain.cuh) where they fit
   ncclComm_t comm = nullptr;
   int world = 1, rank = 0;
   NvlState nvl;            // NVLink peer-memory all-reduce for the latency-bound exchanges (comm_nvl.cuh)

@@ -258,6 +258,36 @@ __device__ __forceinline__ void bn_update_running(const BnRef& bn, int npass, fl
 
 __device__ __forceinline__ float act_lrelu(float x, float slope) { return x > 0.f ? x : x * slope; }
 
+// Epilogue pieces shared by gemm_mn_kernel and the fused row-tile chains (chain.cuh), which must reproduce its results bit
+// for bit: one definition of each expression, so the two cannot drift apart.
+// EP_LINEAR: bias of output feature n with the one-hot label column folded in (scale = 1/sigma or 1)
+__device__ __forceinline__ float ep_bias(const float* bias, const float* wlabel, int ldwl, int n, float scale) {
+  float b = bias ? bias[n] : 0.f;
+  if (wlabel) b += scale * wlabel[(size_t)n * ldwl];
+  return b;
+}
+__device__ __forceinline__ float ep_linear(float acc, float scale, float b) { return fmaf(acc, scale, b); }
+__device__ __forceinline__ float ep_act(float y, int act, float slope) {
+  if (act == ACT_LRELU) return act_lrelu(y, slope);
+  if (act == ACT_RELU) return fmaxf(y, 0.f);
+  if (act == ACT_SIGMOID) return 1.0f / (1.0f + expf(-y));
+  return y;
+}
+__device__ __forceinline__ float ep_dropout(float y, unsigned char keep, float keep_inv) { return keep ? y * keep_inv : 0.f; }
+// EP_DACT: input gradient of a Linear -> gradient w.r.t. the pre-activation of the layer below (dropout, then activation)
+__device__ __forceinline__ float ep_keep(unsigned char keep, float keep_inv) { return keep ? keep_inv : 0.f; }
+__device__ __forceinline__ float ep_dact(float acc, float scale, float keep, float a_prev, float neg) {
+  const float d = acc * scale * keep;
+  return a_prev > 0.f ? d : d * neg;
+}
+// ((p0 + p1) + p2) + p3: the four k-group partials of one output element, in this order
+__device__ __forceinline__ float4 ksum4(float4 v, float4 w1, float4 w2, float4 w3) {
+  v.x += w1.x; v.y += w1.y; v.z += w1.z; v.w += w1.w;
+  v.x += w2.x; v.y += w2.y; v.z += w2.z; v.w += w2.w;
+  v.x += w3.x; v.y += w3.y; v.z += w3.z; v.w += w3.w;
+  return v;
+}
+
 // Loads 4 consecutive batch rows (m..m+3) of feature row r of an operand, transformed; rows >= M and
 // feature rows >= o.rows read as 0.
 // Operand staging is split in two so that global loads stay in flight across the FFMA block: load_raw only
@@ -497,12 +527,8 @@ __global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_mn_kernel(const GemmArgs
   float acc[4][4];
 #pragma unroll
   for (int j = 0; j < 4; ++j) {
-    float4 v = ld4(part + (size_t)(tn + j) * RED_LD + tm);
-#pragma unroll
-    for (int q = 1; q < 4; ++q) {
-      const float4 w = ld4(part + ((size_t)q * TBN + tn + j) * RED_LD + tm);
-      v.x += w.x; v.y += w.y; v.z += w.z; v.w += w.w;
-    }
+    const float4 v = ksum4(ld4(part + (size_t)(tn + j) * RED_LD + tm), ld4(part + ((size_t)1 * TBN + tn + j) * RED_LD + tm),
+                           ld4(part + ((size_t)2 * TBN + tn + j) * RED_LD + tm), ld4(part + ((size_t)3 * TBN + tn + j) * RED_LD + tm));
     acc[0][j] = v.x; acc[1][j] = v.y; acc[2][j] = v.z; acc[3][j] = v.w;
   }
 
@@ -523,10 +549,9 @@ __global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_mn_kernel(const GemmArgs
     if (nvalid) {
       const size_t off = (size_t)n * g.ld + m;
       if (EK == EP_LINEAR) {
-        float b = g.bias ? g.bias[n] : 0.f;
-        if (g.wlabel) b += scale * g.wlabel[(size_t)n * g.ldwl];
+        const float b = ep_bias(g.bias, g.wlabel, g.ldwl, n, scale);
 #pragma unroll
-        for (int i = 0; i < 4; ++i) y[i] = fmaf(y[i], scale, b);
+        for (int i = 0; i < 4; ++i) y[i] = ep_linear(y[i], scale, b);
         if (g.kl_acc) {
 #pragma unroll
           for (int i = 0; i < 4; ++i)
@@ -538,22 +563,14 @@ __global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_mn_kernel(const GemmArgs
           for (int i = 0; i < 4; ++i)
             if (rowv[i]) { s1 += (double)y[i]; s2 += (double)y[i] * (double)y[i]; }
         }
-        if (g.act == ACT_LRELU) {
 #pragma unroll
-          for (int i = 0; i < 4; ++i) y[i] = act_lrelu(y[i], g.slope);
-        } else if (g.act == ACT_RELU) {
-#pragma unroll
-          for (int i = 0; i < 4; ++i) y[i] = fmaxf(y[i], 0.f);
-        } else if (g.act == ACT_SIGMOID) {
-#pragma unroll
-          for (int i = 0; i < 4; ++i) y[i] = 1.0f / (1.0f + expf(-y[i]));
-        }
+        for (int i = 0; i < 4; ++i) y[i] = ep_act(y[i], g.act, g.slope);
         if (g.mask) {
           const uchar4 mk = *reinterpret_cast<const uchar4*>(g.mask + (long long)pass * g.smask + off);
-          y[0] = mk.x ? y[0] * g.keep_inv : 0.f;
-          y[1] = mk.y ? y[1] * g.keep_inv : 0.f;
-          y[2] = mk.z ? y[2] * g.keep_inv : 0.f;
-          y[3] = mk.w ? y[3] * g.keep_inv : 0.f;
+          y[0] = ep_dropout(y[0], mk.x, g.keep_inv);
+          y[1] = ep_dropout(y[1], mk.y, g.keep_inv);
+          y[2] = ep_dropout(y[2], mk.z, g.keep_inv);
+          y[3] = ep_dropout(y[3], mk.w, g.keep_inv);
         }
         if (g.osum) {
 #pragma unroll
@@ -581,17 +598,14 @@ __global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_mn_kernel(const GemmArgs
         float keep[4] = {1.f, 1.f, 1.f, 1.f};
         if (g.mask) {
           const uchar4 mk = *reinterpret_cast<const uchar4*>(g.mask + (long long)pass * g.smask + off);
-          keep[0] = mk.x ? g.keep_inv : 0.f;
-          keep[1] = mk.y ? g.keep_inv : 0.f;
-          keep[2] = mk.z ? g.keep_inv : 0.f;
-          keep[3] = mk.w ? g.keep_inv : 0.f;
+          keep[0] = ep_keep(mk.x, g.keep_inv);
+          keep[1] = ep_keep(mk.y, g.keep_inv);
+          keep[2] = ep_keep(mk.z, g.keep_inv);
+          keep[3] = ep_keep(mk.w, g.keep_inv);
         }
         const float neg = (g.act == ACT_LRELU) ? g.slope : 0.f;
 #pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          float d = y[i] * scale * keep[i];
-          y[i] = aa[i] > 0.f ? d : d * neg;
-        }
+        for (int i = 0; i < 4; ++i) y[i] = ep_dact(y[i], scale, keep[i], aa[i], neg);
         st4(g.Y + (long long)pass * g.sY + off, make_float4(y[0], y[1], y[2], y[3]));
       } else if (EK == EP_STORE) {
         float* dst = g.Y + (long long)pass * g.sY + off;

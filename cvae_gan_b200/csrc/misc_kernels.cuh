@@ -65,22 +65,22 @@ constexpr int LN_ROWS = 32;
 constexpr int LN_MAXF = 32;        // features per thread (C <= 256: every width the reference's formulas give up to F = 512)
 constexpr int LN_MAXF_WIDE = 64;   // second instantiation for the widened model (C <= 512, CvgConfig.hidden)
 
-template <int MAXF>
-__global__ void __launch_bounds__(256) ln_fwd_kernel(const LnArgs g) {
-  __shared__ float red[8][LN_ROWS];
+// The per-row body, shared with the fused classifier chain (chain.cuh): the thread of (lane, warp w) owns row `lane` of a
+// 32-row tile and features [w * C/8, (w + 1) * C/8); all 256 threads of the CTA call it.  load_h(c) reads the row's pre-LN
+// value of feature c, store_a(c, a) takes its output (valid rows only).
+template <int MAXF, class LoadH, class StoreA>
+__device__ __forceinline__ void ln_fwd_row(int C, bool valid, float eps, const float* gam, const float* bet, const uint8_t* mk,
+                                           size_t ldm, float keep_inv, float (*red)[LN_ROWS], LoadH load_h, StoreA store_a,
+                                           float& mean, float& rstd) {
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-  const int m = blockIdx.x * LN_ROWS + lane;
-  const int pass = blockIdx.y;
-  const bool valid = m < g.M;
-  const int fpt = (g.C + 7) / 8;            // features per thread
+  const int fpt = (C + 7) / 8;            // features per thread
   const int c0 = w * fpt;
-  const float* h = g.h + (long long)pass * g.sh + (valid ? m : 0);
   float v[MAXF];
   float s = 0.f;
 #pragma unroll
   for (int i = 0; i < MAXF; ++i) {
     const int c = c0 + i;
-    v[i] = (i < fpt && c < g.C && valid) ? h[(size_t)c * g.ld] : 0.f;
+    v[i] = (i < fpt && c < C && valid) ? load_h(c) : 0.f;
     s += v[i];
   }
   red[w][lane] = s;
@@ -88,33 +88,48 @@ __global__ void __launch_bounds__(256) ln_fwd_kernel(const LnArgs g) {
   float tot = 0.f;
 #pragma unroll
   for (int k = 0; k < 8; ++k) tot += red[k][lane];
-  const float mean = tot / (float)g.C;
+  mean = tot / (float)C;
   __syncthreads();
   float q = 0.f;
 #pragma unroll
   for (int i = 0; i < MAXF; ++i) {
     const int c = c0 + i;
-    if (i < fpt && c < g.C) { const float d = v[i] - mean; q = fmaf(d, d, q); }
+    if (i < fpt && c < C) { const float d = v[i] - mean; q = fmaf(d, d, q); }
   }
   red[w][lane] = q;
   __syncthreads();
   tot = 0.f;
 #pragma unroll
   for (int k = 0; k < 8; ++k) tot += red[k][lane];
-  const float rstd = 1.0f / sqrtf(tot / (float)g.C + g.eps);
+  rstd = 1.0f / sqrtf(tot / (float)C + eps);
   if (!valid) return;
-  float* a = g.a + (long long)pass * g.sa + m;
-  const uint8_t* mk = g.mask ? g.mask + (long long)pass * g.smask + m : nullptr;
 #pragma unroll
   for (int i = 0; i < MAXF; ++i) {
     const int c = c0 + i;
-    if (i < fpt && c < g.C) {
-      float n = (v[i] - mean) * rstd * g.g[c] + g.b[c];
+    if (i < fpt && c < C) {
+      float n = (v[i] - mean) * rstd * gam[c] + bet[c];
       n = fmaxf(n, 0.f);
-      if (mk) n = mk[(size_t)c * g.ld] ? n * g.keep_inv : 0.f;
-      a[(size_t)c * g.ld] = n;
+      if (mk) n = mk[(size_t)c * ldm] ? n * keep_inv : 0.f;
+      store_a(c, n);
     }
   }
+}
+
+template <int MAXF>
+__global__ void __launch_bounds__(256) ln_fwd_kernel(const LnArgs g) {
+  __shared__ float red[8][LN_ROWS];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const int m = blockIdx.x * LN_ROWS + lane;
+  const int pass = blockIdx.y;
+  const bool valid = m < g.M;
+  const float* h = g.h + (long long)pass * g.sh + (valid ? m : 0);
+  float* a = g.a + (long long)pass * g.sa + m;
+  const uint8_t* mk = g.mask ? g.mask + (long long)pass * g.smask + m : nullptr;
+  float mean, rstd;
+  ln_fwd_row<MAXF>(
+      g.C, valid, g.eps, g.g, g.b, mk, g.ld, g.keep_inv, red, [&](int c) { return h[(size_t)c * g.ld]; },
+      [&](int c, float n) { a[(size_t)c * g.ld] = n; }, mean, rstd);
+  if (!valid) return;
   if (g.rs && w == 0) {
     float* rs = g.rs + (long long)pass * g.srs;
     rs[m] = mean;
@@ -133,31 +148,25 @@ struct LnBwdArgs {
   float* dg; float* db;                // null -> skipped
 };
 
-// The affine gradients are summed in fixed point in `acc` ([2C] int64, det_fix: exact, so independent of the block order);
-// the last block (ticket on `cnt`) converts them, adds them to dg / db and clears `acc` and `cnt` (like gemm_dw_kernel).
-template <int MAXF>
-__global__ void __launch_bounds__(256) ln_bwd_kernel(const LnBwdArgs g, unsigned long long* acc, unsigned* cnt) {
-  __shared__ float red1[8][LN_ROWS], red2[8][LN_ROWS];
+// The per-row body, shared with the fused classifier chain (chain.cuh); thread mapping as ln_fwd_row.  load_dn(c) / load_h(c)
+// read the row's dL/dn and pre-LN value of feature c, store_dh(c, v) takes dL/dh (valid rows only).  acc != null: the 32-row
+// sums of the affine gradients go into it in fixed point, [dgamma (C) | dbeta (C)].
+template <int MAXF, class LoadDn, class LoadH, class StoreDh>
+__device__ __forceinline__ void ln_bwd_row(int C, bool valid, float mean, float rstd, const float* gam, float (*red1)[LN_ROWS],
+                                           float (*red2)[LN_ROWS], LoadDn load_dn, LoadH load_h, StoreDh store_dh,
+                                           unsigned long long* acc) {
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-  const int m = blockIdx.x * LN_ROWS + lane;
-  const int pass = blockIdx.y;
-  const bool valid = m < g.M;
-  const int mm = valid ? m : 0;
-  const int fpt = (g.C + 7) / 8;
+  const int fpt = (C + 7) / 8;
   const int c0 = w * fpt;
-  const float* h = g.h + (long long)pass * g.sh + mm;
-  float* dn = g.dn + (long long)pass * g.sdn + mm;
-  const float* rs = g.rs + (long long)pass * g.srs;
-  const float mean = rs[mm], rstd = rs[g.ld + mm];
   float xh[MAXF], d[MAXF];
   float s1 = 0.f, s2 = 0.f;
 #pragma unroll
   for (int i = 0; i < MAXF; ++i) {
     const int c = c0 + i;
-    const bool on = i < fpt && c < g.C && valid;
-    xh[i] = on ? (h[(size_t)c * g.ld] - mean) * rstd : 0.f;
-    d[i] = on ? dn[(size_t)c * g.ld] : 0.f;
-    const float dx = on ? d[i] * g.g[c] : 0.f;
+    const bool on = i < fpt && c < C && valid;
+    xh[i] = on ? (load_h(c) - mean) * rstd : 0.f;
+    d[i] = on ? load_dn(c) : 0.f;
+    const float dx = on ? d[i] * gam[c] : 0.f;
     s1 += dx;
     s2 = fmaf(dx, xh[i], s2);
   }
@@ -167,22 +176,40 @@ __global__ void __launch_bounds__(256) ln_bwd_kernel(const LnBwdArgs g, unsigned
   s1 = 0.f; s2 = 0.f;
 #pragma unroll
   for (int k = 0; k < 8; ++k) { s1 += red1[k][lane]; s2 += red2[k][lane]; }
-  s1 /= (float)g.C;
-  s2 /= (float)g.C;
+  s1 /= (float)C;
+  s2 /= (float)C;
 #pragma unroll
   for (int i = 0; i < MAXF; ++i) {
     const int c = c0 + i;
-    const bool on = i < fpt && c < g.C;       // warp-uniform
+    const bool on = i < fpt && c < C;       // warp-uniform
     if (!on) continue;
-    if (valid) dn[(size_t)c * g.ld] = rstd * (d[i] * g.g[c] - s1 - xh[i] * s2);
-    if (g.dg) {
+    if (valid) store_dh(c, rstd * (d[i] * gam[c] - s1 - xh[i] * s2));
+    if (acc) {
       const float a = warp_sum(d[i] * xh[i]), b = warp_sum(d[i]);
       if (lane == 0) {
         atomicAdd(acc + c, det_fix(a));
-        atomicAdd(acc + g.C + c, det_fix(b));
+        atomicAdd(acc + C + c, det_fix(b));
       }
     }
   }
+}
+
+// The affine gradients are summed in fixed point in `acc` ([2C] int64, det_fix: exact, so independent of the block order);
+// the last block (ticket on `cnt`) converts them, adds them to dg / db and clears `acc` and `cnt` (like gemm_dw_kernel).
+template <int MAXF>
+__global__ void __launch_bounds__(256) ln_bwd_kernel(const LnBwdArgs g, unsigned long long* acc, unsigned* cnt) {
+  __shared__ float red1[8][LN_ROWS], red2[8][LN_ROWS];
+  const int lane = threadIdx.x & 31;
+  const int m = blockIdx.x * LN_ROWS + lane;
+  const int pass = blockIdx.y;
+  const bool valid = m < g.M;
+  const int mm = valid ? m : 0;
+  const float* h = g.h + (long long)pass * g.sh + mm;
+  float* dn = g.dn + (long long)pass * g.sdn + mm;
+  const float* rs = g.rs + (long long)pass * g.srs;
+  ln_bwd_row<MAXF>(
+      g.C, valid, rs[mm], rs[g.ld + mm], g.g, red1, red2, [&](int c) { return dn[(size_t)c * g.ld]; },
+      [&](int c) { return h[(size_t)c * g.ld]; }, [&](int c, float v) { dn[(size_t)c * g.ld] = v; }, g.dg ? acc : nullptr);
   if (!g.dg) return;
   __threadfence();
   __syncthreads();
@@ -224,25 +251,30 @@ struct CeArgs {
   const long long* labels = nullptr;   // per-row targets (downstream Classifier.fit); null -> the shared `label`
 };
 
+// One row: K logits `ldl` apart in, K logit gradients `ldd` apart out; returns the row's negative log-likelihood.  Shared with
+// the fused classifier chain (chain.cuh).
+__device__ __forceinline__ double ce_row(const float* l, size_t ldl, float* d, size_t ldd, int K, int tgt, float coef) {
+  float mx = -INFINITY;
+  for (int k = 0; k < K; ++k) mx = fmaxf(mx, l[(size_t)k * ldl]);
+  float s = 0.f;
+  for (int k = 0; k < K; ++k) s += expf(l[(size_t)k * ldl] - mx);
+  const float lse = logf(s);
+  const double nll = -(double)(l[(size_t)tgt * ldl] - mx - lse);
+  for (int k = 0; k < K; ++k) {
+    const float p = expf(l[(size_t)k * ldl] - mx - lse);
+    d[(size_t)k * ldd] = (p - (k == tgt ? 1.f : 0.f)) * coef;
+  }
+  return nll;
+}
+
 __global__ void ce_kernel(const CeArgs g) {
   const int m = blockIdx.x * blockDim.x + threadIdx.x;
   const int pass = blockIdx.y;
   double nll = 0.0;
   if (m < g.M) {
-    const float* l = g.logits + (long long)pass * g.sl + m;
-    float mx = -INFINITY;
-    for (int k = 0; k < g.K; ++k) mx = fmaxf(mx, l[(size_t)k * g.ld]);
-    float s = 0.f;
-    for (int k = 0; k < g.K; ++k) s += expf(l[(size_t)k * g.ld] - mx);
-    const float lse = logf(s);
     const int tgt = g.labels ? (int)g.labels[m] : g.label;
-    nll = -(double)(l[(size_t)tgt * g.ld] - mx - lse);
-    float* d = g.dlogits + (long long)pass * g.sd + m;
     const float coef = g.ctl ? g.coef * g.ctl->lambda_class : g.coef;
-    for (int k = 0; k < g.K; ++k) {
-      const float p = expf(l[(size_t)k * g.ld] - mx - lse);
-      d[(size_t)k * g.ld] = (p - (k == tgt ? 1.f : 0.f)) * coef;
-    }
+    nll = ce_row(g.logits + (long long)pass * g.sl + m, g.ld, g.dlogits + (long long)pass * g.sd + m, g.ld, g.K, tgt, coef);
   }
   nll = warp_sum_d(nll);
   if ((threadIdx.x & 31) == 0 && nll != 0.0) atomicAdd(g.loss + pass, nll);

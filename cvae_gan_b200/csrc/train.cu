@@ -4,6 +4,7 @@
 #include <dlfcn.h>
 #include <math.h>
 
+#include "chain.cuh"
 #include "engine.cuh"
 #include "mega.cuh"
 
@@ -707,12 +708,95 @@ int fwd_classifier(Engine& e, const float* xin, long long sxin, int npass, bool 
 }
 
 // ------------------------------------------------------------------------------------------------
+// fused row-tile chains of the D and C steps (chain.cuh)
+// ------------------------------------------------------------------------------------------------
+// Used where the layer kernels would otherwise run stand-alone (the step-program kernel records layer ops) and at the widths
+// the chains are built for; the widened model (CvgConfig.hidden) keeps the layer kernels.
+static bool chain_usable(const Engine& e, int net) {
+  if (!e.chain || e.mk.recording) return false;
+  const int* h = net == CVG_NET_DISCRIMINATOR ? e.dh : e.ch;
+  return h[0] == CH_H0 && h[1] == CH_H1 && h[2] == CH_H2 && e.F <= CH_MAX_IN && e.K <= CH_MAX_K;
+}
+
+// After a chain the weight gradients of the four layers are independent of each other: the largest (layer 1) runs on the
+// caller's stream, the others beside it on the side streams (each stream has its own deterministic-reduction slot).
+static cudaStream_t chain_dw_stream(Engine& e, int l, cudaStream_t st) { return l == 1 ? st : fork_to(e, l == 2 ? 1 : 0, st); }
+
+// Critic forward (score sums into loss[L_DREAL + pass]) and input gradients from the per-pass seed, both passes, one launch.
+static int launch_critic_chain(Engine& e, long long sx, int label, int M, const float* seed, cudaStream_t st) {
+  const int net = CVG_NET_DISCRIMINATOR;
+  const Workspace& w = e.ws;
+  CriticChainArgs a;
+  a.M = M; a.ld = w.ld; a.F = e.F;
+  a.x = w.xT; a.sx = sx;
+  double flops = 0.0;
+  for (int l = 0; l < 4; ++l) {
+    const LinearP& p = lin(e, net, l);
+    a.W[l] = e.P(net, p.w); a.ldw[l] = p.in; a.b[l] = e.P(net, p.b);
+    flops += 2.0 * ((l == 0) ? e.F : p.in) * p.out + (l > 0 ? 2.0 * p.in * p.out : 0.0);
+  }
+  a.wlabel = label_column(e, net, lin(e, net, 0), e.F, label);
+  a.ldwl = lin(e, net, 0).in;
+  a.inv_sigma = w.sn_inv_sigma;
+  a.m1 = w.d_m1; a.m2 = w.d_m2;
+  a.keep_inv = 1.0f / (1.0f - e.cfg.dropout_p);
+  a.slope = e.cfg.lrelu_slope;
+  for (int i = 0; i < 3; ++i) { a.a[i] = w.d_a[i]; a.g[i] = w.d_g[i]; }
+  a.s = w.d_s;
+  a.osum = w.loss + L_DREAL;
+  a.seed[0] = seed[0]; a.seed[1] = seed[1];
+  const dim3 grid(2 * ((M + TBM - 1) / TBM), 2);
+  prof_begin(e, 3, flops * 2 * M, st);
+  critic_chain_kernel<<<grid, CH_THREADS, critic_chain_smem(e.F), st>>>(a);
+  prof_end(e, st);
+  CVG_LAUNCH_CHECK();
+  return 0;
+}
+
+// Classifier forward, cross-entropy with the step's label (loss[L_CE0 + pass]), input gradients with the LayerNorm backward
+// and its affine gradients, both passes, one launch.
+static int launch_classifier_chain(Engine& e, long long sx, int label, int M, float coef, cudaStream_t st) {
+  const int net = CVG_NET_CLASSIFIER;
+  const Workspace& w = e.ws;
+  ClassifierChainArgs a;
+  a.M = M; a.ld = w.ld; a.F = e.F; a.K = e.K; a.label = label;
+  a.x = w.xT; a.sx = sx;
+  double flops = 0.0;
+  for (int l = 0; l < 4; ++l) {
+    const LinearP& p = lin(e, net, l);
+    a.W[l] = e.P(net, p.w); a.b[l] = e.P(net, p.b);
+    flops += 2.0 * p.in * p.out * (l > 0 ? 2.0 : 1.0);
+  }
+  const LinearP& p1 = lin(e, net, 1);
+  a.gamma = e.P(net, p1.gamma); a.beta = e.P(net, p1.beta);
+  a.ln_eps = e.cfg.ln_eps;
+  a.m1 = w.c_m1; a.m2 = w.c_m2;
+  a.keep_inv = 1.0f / (1.0f - e.cfg.dropout_p);
+  a.a1 = w.c_a1; a.h2 = w.c_h2; a.a2 = w.c_a2; a.rs = w.c_rs; a.a3 = w.c_a3; a.logit = w.c_logit; a.dlogit = w.c_dlogit;
+  for (int i = 0; i < 3; ++i) a.g[i] = w.c_g[i];
+  a.coef = coef;
+  a.loss = w.loss + L_CE0;
+  a.dgamma = e.G(net, p1.gamma); a.dbeta = e.G(net, p1.beta);
+  const int slot = det_slot(e, st);
+  if (2LL * CH_H1 > e.ws.det_acc_n) CVG_FAIL("internal: LayerNorm backward exceeds the deterministic-reduction slots");
+  a.acc = e.ws.det_acc[slot]; a.cnt = e.ws.det_cnt[slot];
+  const dim3 grid(2 * ((M + TBM - 1) / TBM), 2);
+  prof_begin(e, 3, flops * 2 * M, st);
+  classifier_chain_kernel<<<grid, CH_THREADS, classifier_chain_smem(e.F, e.K), st>>>(a);
+  prof_end(e, st);
+  CVG_LAUNCH_CHECK();
+  return 0;
+}
+
+// ------------------------------------------------------------------------------------------------
 // backward passes
 // ------------------------------------------------------------------------------------------------
 // critic backward.  seed[pass] = dL/dscore (constant over rows).  want_dw: accumulate per-pass raw
 // gradients into ws.sn_G (+ bias grads into the grad buffer).  want_dx: write dL/dx into ws.dx.
+// dw_only: a fused chain (chain.cuh) has produced the input gradients; only the weight gradients are launched, spread over
+// the streams (chain_dw_stream).
 static int bwd_critic(Engine& e, const float* xin, long long sxin, int npass, int label, int M, const float* seed,
-                      bool want_dw, bool want_dx, cudaStream_t st) {
+                      bool want_dw, bool want_dx, cudaStream_t st, bool dw_only = false) {
   const int net = CVG_NET_DISCRIMINATOR;
   const Workspace& w = e.ws;
   const size_t ld = w.ld;
@@ -730,7 +814,8 @@ static int bwd_critic(Engine& e, const float* xin, long long sxin, int npass, in
     if (want_dw) {
       // OP_CONST carries one value: run the two passes of layer 4 as separate launches
       const int reps = (l == 3 && npass > 1) ? npass : 1;
-      const cudaStream_t sw = fork_to(e, 0, st);      // beside the input-gradient chain: both only read dY of layer l
+      // beside the input-gradient chain: both only read dY of layer l
+      const cudaStream_t sw = dw_only ? chain_dw_stream(e, l, st) : fork_to(e, 0, st);
       for (int r = 0; r < reps; ++r) {
         if (r > 0) CVG_PAR(e);
         DwArgs d = base_dw(e, M, (float)M, reps > 1 ? 1 : npass);
@@ -750,6 +835,7 @@ static int bwd_critic(Engine& e, const float* xin, long long sxin, int npass, in
         CVG_TRY(launch_dw(e, d, sw));
       }
     }
+    if (dw_only) continue;
     if (l == 0 && !want_dx) break;
     GemmArgs g = base_args(e, M, (float)M, npass);
     g.R = p.out;
@@ -791,8 +877,9 @@ static int bwd_critic(Engine& e, const float* xin, long long sxin, int npass, in
 
 // classifier backward from ws.c_dlogit.
 // dx_after: a stream whose enqueued work writes ws.dx first (the critic's backward, when this one runs beside it).
+// dw_only: as bwd_critic.
 static int bwd_classifier(Engine& e, const float* xin, long long sxin, int npass, int M, bool want_dw, bool want_dx,
-                          bool dx_accumulate, cudaStream_t st, cudaStream_t dx_after = nullptr) {
+                          bool dx_accumulate, cudaStream_t st, cudaStream_t dx_after = nullptr, bool dw_only = false) {
   const int net = CVG_NET_CLASSIFIER;
   const Workspace& w = e.ws;
   const size_t ld = w.ld;
@@ -819,8 +906,9 @@ static int bwd_classifier(Engine& e, const float* xin, long long sxin, int npass
       d.sdW = 0;
       d.ldw = p.in;
       d.db = e.G(net, p.b);
-      CVG_TRY(launch_dw(e, d, fork_to(e, 0, st)));
+      CVG_TRY(launch_dw(e, d, dw_only ? chain_dw_stream(e, l, st) : fork_to(e, 0, st)));
     }
+    if (dw_only) continue;
     if (l == 0 && !want_dx) break;
     if (l == 0 && dx_after) {
       wait_for(e, st, dx_after);
@@ -1204,9 +1292,14 @@ int step_d(Engine& e, const float* x_real, int label, int B, const CvgNoise* nz,
   if (!e.hoist_x) CVG_TRY(fwd_generator(e, 1, true, false, label, B, Bg_bn, local_bn, st));
   join_sides(e, st);
   const long long sx = (e.hoist_x ? e.hoist_x : w.g_out) - w.xT;  // pass 0 reads xT, pass 1 reads G(z)
-  CVG_TRY(fwd_critic(e, w.xT, sx, 2, label, B, w.loss + L_DREAL, st));
   const float seedv[2] = {-1.0f / Bg, 1.0f / Bg};   // d_loss = -mean D(real) + mean D(fake)
-  CVG_TRY(bwd_critic(e, w.xT, sx, 2, label, B, seedv, true, false, st));
+  if (chain_usable(e, D)) {
+    CVG_TRY(launch_critic_chain(e, sx, label, B, seedv, st));
+    CVG_TRY(bwd_critic(e, w.xT, sx, 2, label, B, seedv, true, false, st, true));
+  } else {
+    CVG_TRY(fwd_critic(e, w.xT, sx, 2, label, B, w.loss + L_DREAL, st));
+    CVG_TRY(bwd_critic(e, w.xT, sx, 2, label, B, seedv, true, false, st));
+  }
   join_sides(e, st);
   {
     SnGradArgs a;
@@ -1272,16 +1365,21 @@ int step_c(Engine& e, const float* x_real, int label, int B, const CvgNoise* nz,
   if (!e.hoist_x) CVG_TRY(fwd_generator(e, 1, true, false, label, B, Bg_bn, local_bn, st));
   join_sides(e, st);
   const long long sx = (e.hoist_x ? e.hoist_x : w.g_out) - w.xT;
-  CVG_TRY(fwd_classifier(e, w.xT, sx, 2, true, B, st));
-  CeArgs c;
-  c.M = B; c.ld = w.ld; c.K = e.K; c.npass = 2; c.label = label;
-  c.logits = w.c_logit; c.sl = (long long)e.K * ld;
-  c.dlogits = w.c_dlogit; c.sd = (long long)e.K * ld;
-  c.coef = 1.0f / Bg;
-  c.ctl = nullptr;
-  c.loss = w.loss + L_CE0;
-  CVG_TRY(emit_ce(e, c, B, 2, st));
-  CVG_TRY(bwd_classifier(e, w.xT, sx, 2, B, true, false, false, st));
+  if (chain_usable(e, C)) {
+    CVG_TRY(launch_classifier_chain(e, sx, label, B, 1.0f / Bg, st));
+    CVG_TRY(bwd_classifier(e, w.xT, sx, 2, B, true, false, false, st, nullptr, true));
+  } else {
+    CVG_TRY(fwd_classifier(e, w.xT, sx, 2, true, B, st));
+    CeArgs c;
+    c.M = B; c.ld = w.ld; c.K = e.K; c.npass = 2; c.label = label;
+    c.logits = w.c_logit; c.sl = (long long)e.K * ld;
+    c.dlogits = w.c_dlogit; c.sd = (long long)e.K * ld;
+    c.coef = 1.0f / Bg;
+    c.ctl = nullptr;
+    c.loss = w.loss + L_CE0;
+    CVG_TRY(emit_ce(e, c, B, 2, st));
+    CVG_TRY(bwd_classifier(e, w.xT, sx, 2, B, true, false, false, st));
+  }
   CVG_TRY(finish_step(e, 1 << C, 1, B, flags, loss_out, st));
   return prog.finish(st);
 }
@@ -1706,6 +1804,9 @@ int visit(Engine& e, int label, int B, int64_t B_global, const float* class_rows
 void set_all_kernel_attributes() {
   mk_set_kernel_attributes();
   cudaFuncSetAttribute(sn_power_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SN_W_SMEM_MAX);
+  cudaFuncSetAttribute(critic_chain_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)critic_chain_smem(CH_MAX_IN));
+  cudaFuncSetAttribute(classifier_chain_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                       (int)classifier_chain_smem(CH_MAX_IN, CH_MAX_K));
   // cudaFuncSetAttribute is done once, eagerly, so that nothing but launches happens during graph capture
 #define CVG_MN_ATTR(W, A, E) cudaFuncSetAttribute(gemm_mn_kernel<W, A, E>, cudaFuncAttributeMaxDynamicSharedMemorySize, 112 * 1024);
   CVG_MN_ATTR(true, OP_PLAIN, EP_LINEAR) CVG_MN_ATTR(true, OP_BN_ACT, EP_LINEAR) CVG_MN_ATTR(true, OP_REPARAM, EP_LINEAR)
