@@ -114,7 +114,7 @@ int cvg_create(const CvgConfig* cfg, CvgHandle** out) {
     const char* off = getenv("CVG_STREAMS");
     ms.on = !(off && off[0] == '0');
     bool ok = true;
-    for (int i = 0; i < 2 && ok; ++i) ok = cudaStreamCreateWithFlags(&ms.s[i], cudaStreamNonBlocking) == cudaSuccess;
+    for (int i = 0; i < SIDE_STREAMS && ok; ++i) ok = cudaStreamCreateWithFlags(&ms.s[i], cudaStreamNonBlocking) == cudaSuccess;
     for (int i = 0; i < SIDE_EVENTS && ok; ++i) ok = cudaEventCreateWithFlags(&ms.ev[i], cudaEventDisableTiming) == cudaSuccess;
     for (int i = 0; i < 4 && ok; ++i) ok = cudaEventCreateWithFlags(&ms.layer[i], cudaEventDisableTiming) == cudaSuccess;
     if (!ok) {
@@ -129,7 +129,7 @@ int cvg_create(const CvgConfig* cfg, CvgHandle** out) {
 
 void cvg_destroy(CvgHandle* h) {
   if (!h) return;
-  for (int i = 0; i < 2; ++i)
+  for (int i = 0; i < SIDE_STREAMS; ++i)
     if (h->e.ms.s[i]) cudaStreamDestroy(h->e.ms.s[i]);
   for (int i = 0; i < SIDE_EVENTS; ++i)
     if (h->e.ms.ev[i]) cudaEventDestroy(h->e.ms.ev[i]);
@@ -501,6 +501,7 @@ int cvg_debug_set(CvgHandle* h, const char* key, int value) {
   else if (k == "hoist") e.hoist = value != 0;
   else if (k == "streams") e.ms.on = value != 0;
   else if (k == "chain") e.chain = value != 0;      // 0: the D / C steps run the layer kernels (the chains' reference)
+  else if (k == "eg_split") e.eg_split = value != 0;   // 0: the E/G step's generator backward runs both passes per launch
   else if (k == "fuse_stats") e.nvl.fuse = value != 0;
   else CVG_FAIL("cvg_debug_set: unknown key");
   return 0;

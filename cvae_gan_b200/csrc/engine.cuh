@@ -13,6 +13,7 @@ constexpr int HOIST_MAX = 16;  // generator passes one hoisted forward can hold 
 constexpr int STAT_C = 1024;   // max features of a BatchNorm layer (stats slots are [2][STAT_C])
 
 constexpr int DET_MAX_PASS = 4;   // passes per launch the deterministic-reduction slots are sized for
+constexpr int SIDE_STREAMS = 3;   // streams beside the caller's (SideStreams)
 
 // feature-major workspace (all float matrices are [features][ld], two pass slots where noted)
 struct Workspace {
@@ -81,10 +82,10 @@ struct Workspace {
   float* dw_scratch = nullptr;
   long long dw_scratch_floats = 0;
   // stand-alone kernels' deterministic reductions (gemm_dw_kernel, ln_bwd_kernel): fixed-point accumulators and ticket
-  // counters, one set per stream the engine launches on (0: the caller's, 1 / 2: the side streams), since launches on one
+  // counters, one set per stream the engine launches on (0: the caller's, 1 + i: side stream i), since launches on one
   // stream never overlap
-  unsigned long long* det_acc[3] = {};
-  unsigned* det_cnt[3] = {};
+  unsigned long long* det_acc[SIDE_STREAMS + 1] = {};
+  unsigned* det_cnt[SIDE_STREAMS + 1] = {};
   long long det_acc_n = 0;
   int det_cnt_n = 0;
   unsigned int* mk_bar = nullptr;
@@ -146,18 +147,20 @@ struct ProfRec {
   double flops;
 };
 
-// Two extra streams beside the caller's: the stand-alone layer kernels are latency bound at the benchmarked sizes, so
+// Extra streams beside the caller's: the stand-alone layer kernels are latency bound at the benchmarked sizes, so
 // independent ones (weight gradients beside the input-gradient chain, the critic's power iteration and the batch staging
 // beside the noise fill, C beside D in the E/G step) run concurrently.  Fork / join with events, so the work stays
-// capturable in the caller's CUDA graph and ordered with the caller's stream.
+// capturable in the caller's CUDA graph and ordered with the caller's stream.  The third side stream only carries the
+// encoder's weight gradients of the E/G step, whose generator backward runs as two per-pass chains on the caller's stream
+// and side stream 1, with the generator's weight gradients on side stream 0.
 constexpr int SIDE_EVENTS = 32;   // fork / join events, used round-robin (far more than are ever pending at once)
 struct SideStreams {
   bool on = false;
-  cudaStream_t s[2] = {nullptr, nullptr};
+  cudaStream_t s[SIDE_STREAMS] = {};
   cudaEvent_t ev[SIDE_EVENTS] = {};
   cudaEvent_t layer[4] = {};        // E/G step: layer l of the generator's z_prior pass is done (the z_enc pass waits for it)
   unsigned next = 0;
-  bool dirty[2] = {false, false};
+  bool dirty[SIDE_STREAMS] = {};
 };
 
 struct Engine {
@@ -179,6 +182,7 @@ struct Engine {
   unsigned long long step_dcounter = 0;   // visit(): Philox counter values the step being emitted uses (advanced at its end)
   int hoist = 1;                    // CVG_HOIST=0: every step runs its own generator forward
   bool chain = true;                // D / C steps run the critic / classifier as fused row-tile chains (chain.cuh) where they fit
+  bool eg_split = true;             // the E/G step runs the generator backward of its two passes as two chains (train.cu step_g)
   ncclComm_t comm = nullptr;
   int world = 1, rank = 0;
   NvlState nvl;            // NVLink peer-memory all-reduce for the latency-bound exchanges (comm_nvl.cuh)

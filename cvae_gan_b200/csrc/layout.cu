@@ -259,7 +259,7 @@ static size_t carve(const Engine& e, Workspace& w, void* base) {
       }
     w.det_acc_n = std::max((long long)tiles * DET_MAX_PASS * DW_PART, 2LL * cmax);
     w.det_cnt_n = tiles;
-    for (int i = 0; i < 3; ++i) {
+    for (int i = 0; i < SIDE_STREAMS + 1; ++i) {
       w.det_acc[i] = c.take<unsigned long long>((size_t)w.det_acc_n);
       w.det_cnt[i] = c.take<unsigned>((size_t)w.det_cnt_n);
     }

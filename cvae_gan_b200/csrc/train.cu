@@ -266,7 +266,11 @@ int launch_mn(Engine& e, bool wt, const GemmArgs& g_in, cudaStream_t st) {
 }
 
 // the deterministic-reduction slot set of the stream a stand-alone kernel is launched on (Workspace::det_acc)
-static int det_slot(const Engine& e, cudaStream_t st) { return st == e.ms.s[0] ? 1 : st == e.ms.s[1] ? 2 : 0; }
+static int det_slot(const Engine& e, cudaStream_t st) {
+  for (int i = 0; i < SIDE_STREAMS; ++i)
+    if (st == e.ms.s[i]) return 1 + i;
+  return 0;
+}
 
 int launch_dw(Engine& e, const DwArgs& g0, cudaStream_t st) {
   if (e.mk.recording) return mk_push_dw(e, g0);
@@ -397,7 +401,7 @@ static void wait_for(Engine& e, cudaStream_t waiter, cudaStream_t signaller) {
 }
 // `st` continues after everything enqueued on the side streams
 static void join_sides(Engine& e, cudaStream_t st, int only = -1) {
-  for (int i = 0; i < 2; ++i) {
+  for (int i = 0; i < SIDE_STREAMS; ++i) {
     if (!e.ms.dirty[i] || (only >= 0 && only != i)) continue;
     cudaEvent_t ev = e.ms.ev[e.ms.next++ % SIDE_EVENTS];
     cudaEventRecord(ev, e.ms.s[i]);
@@ -973,84 +977,104 @@ struct BnNetBwd {
   bool want_first_dx;      // generator: dL/dz_enc of pass 0 -> encoder head gradient
 };
 
-static int bwd_bn_net(Engine& e, const BnNetBwd& b, int M, float Bg_bn, float kl_coef, bool local_bn, cudaStream_t st) {
+// dY operand of layer l: the gradient w.r.t. the output of its Linear
+static Operand bn_net_dy(const Engine& e, const BnNetBwd& b, int l) {
+  const LinearP& p = lin(e, b.net, l);
+  Operand dy;
+  if (l == 3) {
+    dy.kind = OP_PLAIN; dy.rows = p.out; dy.p = b.top_dy; dy.sp = b.s_top;
+  } else {
+    dy.kind = OP_BN_BWD; dy.rows = p.out;
+    dy.p = b.dy[l]; dy.sp = (long long)p.out * e.ws.ld;
+    dy.h = b.h[l]; dy.sh = (long long)p.out * e.ws.ld;
+    dy.bn = bn_ref(e, b.net, l, false, false);
+  }
+  return dy;
+}
+
+// Input gradient of layer l: dY of layer l - 1 with its batch sums, or, at layer 0 with want_first_dx, the encoder head
+// gradient (pass 0 only).  Nothing at layer 0 otherwise.  only_pass >= 0: that pass alone, in a grid of one pass slot.
+static int bwd_bn_dx(Engine& e, const BnNetBwd& b, int l, int M, float Bg_bn, float kl_coef, bool local_bn, cudaStream_t st,
+                     int only_pass = -1) {
   const Workspace& w = e.ws;
   const size_t ld = w.ld;
   const int net = b.net;
+  const LinearP& p = lin(e, net, l);
+  if (l > 0) {
+    const LinearP& pp = lin(e, net, l - 1);
+    GemmArgs g = base_args(e, M, Bg_bn, b.npass);
+    g.only_pass = only_pass;
+    g.R = p.out;
+    g.N = p.in;
+    g.a = bn_net_dy(e, b, l);
+    g.W = e.P(net, p.w);
+    g.ldw = p.in;
+    g.ekind = EP_DBN;
+    g.prev = b.h[l - 1];
+    g.sprev = (long long)pp.out * ld;
+    g.prev_bn = bn_ref(e, net, l - 1, false, false);
+    g.Y = b.dy[l - 1];
+    g.sY = (long long)pp.out * ld;
+    g.ostats = bst_of(e, net, l - 1);
+    g.sostats = 2 * STAT_C;
+    return launch_mn_stats(e, false, g, b.npass, local_bn, st);
+  }
+  if (!b.want_first_dx) return 0;
+  GemmArgs g = base_args(e, M, Bg_bn, b.npass);
+  g.only_pass = 0;
+  g.R = p.out;
+  g.N = e.Z;
+  g.a = bn_net_dy(e, b, l);
+  g.W = e.P(net, p.w);
+  g.ldw = p.in;
+  g.ekind = EP_REPARAM_BWD;
+  g.mu = w.e_ml;
+  g.lv = w.e_ml + (size_t)e.Z * ld;
+  g.eps = e.mk.recording ? w.z_eps : w.z;
+  g.kl_coef = kl_coef;
+  g.Y = w.e_dml;
+  return launch_mn(e, false, g, st);
+}
+
+// dW, db and the BatchNorm affine gradients of layer l, all passes in one launch
+static int bwd_bn_dw(Engine& e, const BnNetBwd& b, int l, int M, float Bg_bn, bool local_bn, cudaStream_t st) {
+  const int net = b.net;
+  const LinearP& p = lin(e, net, l);
+  DwArgs d = base_dw(e, M, Bg_bn, b.npass);
+  d.N = p.out;
+  d.p = bn_net_dy(e, b, l);
+  if (l == 0) {
+    d.K = b.first_K;
+    d.q = b.first_in;
+    d.label_col = b.label_col;
+  } else {
+    d.K = p.in;
+    d.q.kind = OP_BN_ACT;
+    d.q.rows = p.in;
+    d.q.p = b.h[l - 1];
+    d.q.sp = (long long)p.in * e.ws.ld;
+    d.q.bn = bn_ref(e, net, l - 1, false, false);
+  }
+  d.dW = e.G(net, p.w);
+  d.sdW = 0;
+  d.ldw = p.in;
+  d.db = e.G(net, p.b);
+  if (l < 3) {
+    d.dgamma = e.G(net, p.gamma);
+    d.dbeta = e.G(net, p.beta);
+    // with global BatchNorm the sums are already global: only rank 0 contributes them before the
+    // gradient all-reduce (sum).  With local BatchNorm every rank adds its own.
+    d.add_affine = (e.world <= 1 || local_bn || e.rank == 0) ? 1 : 0;
+  }
+  return launch_dw(e, d, st);
+}
+
+static int bwd_bn_net(Engine& e, const BnNetBwd& b, int M, float Bg_bn, float kl_coef, bool local_bn, cudaStream_t st) {
   for (int l = 3; l >= 0; --l) {
-    const LinearP& p = lin(e, net, l);
-    Operand dy;
-    if (l == 3) {
-      dy.kind = OP_PLAIN; dy.rows = p.out; dy.p = b.top_dy; dy.sp = b.s_top;
-    } else {
-      dy.kind = OP_BN_BWD; dy.rows = p.out;
-      dy.p = b.dy[l]; dy.sp = (long long)p.out * ld;
-      dy.h = b.h[l]; dy.sh = (long long)p.out * ld;
-      dy.bn = bn_ref(e, net, l, false, false);
-    }
-    // ---- dX first: it produces the batch sums the next layer's kernels need -----------------------
-    if (l > 0) {
-      const LinearP& pp = lin(e, net, l - 1);
-      GemmArgs g = base_args(e, M, Bg_bn, b.npass);
-      g.R = p.out;
-      g.N = p.in;
-      g.a = dy;
-      g.W = e.P(net, p.w);
-      g.ldw = p.in;
-      g.ekind = EP_DBN;
-      g.prev = b.h[l - 1];
-      g.sprev = (long long)pp.out * ld;
-      g.prev_bn = bn_ref(e, net, l - 1, false, false);
-      g.Y = b.dy[l - 1];
-      g.sY = (long long)pp.out * ld;
-      g.ostats = bst_of(e, net, l - 1);
-      g.sostats = 2 * STAT_C;
-      CVG_TRY(launch_mn_stats(e, false, g, b.npass, local_bn, st));
-    } else if (b.want_first_dx) {
-      GemmArgs g = base_args(e, M, Bg_bn, b.npass);
-      g.only_pass = 0;
-      g.R = p.out;
-      g.N = e.Z;
-      g.a = dy;
-      g.W = e.P(net, p.w);
-      g.ldw = p.in;
-      g.ekind = EP_REPARAM_BWD;
-      g.mu = w.e_ml;
-      g.lv = w.e_ml + (size_t)e.Z * ld;
-      g.eps = e.mk.recording ? w.z_eps : w.z;
-      g.kl_coef = kl_coef;
-      g.Y = w.e_dml;
-      CVG_TRY(launch_mn(e, false, g, st));
-    }
-    // ---- dW, db, and the BatchNorm affine gradients of this layer ------------------------------------
+    // dX first: it produces the batch sums the next layer's kernels need
+    CVG_TRY(bwd_bn_dx(e, b, l, M, Bg_bn, kl_coef, local_bn, st));
     if (l > 0 || b.want_first_dx) CVG_PAR(e);     // beside the input-gradient op just emitted: both read dY of layer l
-    DwArgs d = base_dw(e, M, Bg_bn, b.npass);
-    d.N = p.out;
-    d.p = dy;
-    if (l == 0) {
-      d.K = b.first_K;
-      d.q = b.first_in;
-      d.label_col = b.label_col;
-    } else {
-      d.K = p.in;
-      d.q.kind = OP_BN_ACT;
-      d.q.rows = p.in;
-      d.q.p = b.h[l - 1];
-      d.q.sp = (long long)p.in * ld;
-      d.q.bn = bn_ref(e, net, l - 1, false, false);
-    }
-    d.dW = e.G(net, p.w);
-    d.sdW = 0;
-    d.ldw = p.in;
-    d.db = e.G(net, p.b);
-    if (l < 3) {
-      d.dgamma = e.G(net, p.gamma);
-      d.dbeta = e.G(net, p.beta);
-      // with global BatchNorm the sums are already global: only rank 0 contributes them before the
-      // gradient all-reduce (sum).  With local BatchNorm every rank adds its own.
-      d.add_affine = (e.world <= 1 || local_bn || e.rank == 0) ? 1 : 0;
-    }
-    CVG_TRY(launch_dw(e, d, fork_to(e, 0, st)));
+    CVG_TRY(bwd_bn_dw(e, b, l, M, Bg_bn, local_bn, fork_to(e, 0, st)));
   }
   return 0;
 }
@@ -1621,6 +1645,15 @@ int step_g(Engine& e, const float* x_real, int label, int B, const CvgNoise* nz,
   //   side 1          : batch staging, G(z_prior), then D(x_fake) forward and backward to x_fake
   //   side 0          : power iteration, then C(x_fake) forward, loss and backward to x_fake (after D's: both add to ws.dx)
   const bool three = !e.mk.recording && e.ms.on && (e.world <= 1 || local_bn || fold_stats(e, local_bn));
+  // The backward continues as two chains, one per generator pass (their BatchNorm sums are per pass, and only pass 0
+  // reaches the encoder):
+  //   caller's stream : seed and generator input gradients of pass 0, the encoder head gradient, the encoder backward
+  //   side 1          : after the critic's and classifier's dx, seed and generator input gradients of pass 1
+  //   side 0          : the generator's weight gradients, each after both passes' dY of its layer (one launch for both
+  //                     passes, so the fixed-point sums are converted once, as with one chain)
+  //   side 2          : the encoder's weight gradients, which must not queue behind the generator's
+  // Only where no BatchNorm sums are exchanged: a folded exchange of one pass cannot yet be told from the other pass's.
+  const bool split = three && e.eg_split && (e.world <= 1 || local_bn);
   join_sides(e, st);      // the previous step's Adam (visit: side stream 0) beside the fill just launched
   if (three) {
     const cudaStream_t sA = fork_to(e, 0, st), sB = fork_to(e, 1, st);
@@ -1643,7 +1676,7 @@ int step_g(Engine& e, const float* x_real, int label, int B, const CvgNoise* nz,
     GenSplit enc;
     enc.only_pass = 0; enc.channel = 0; enc.wait = e.ms.layer;
     CVG_TRY(fwd_generator(e, 2, true, true, label, B, Bg_bn, local_bn, st, nullptr, &enc));
-    join_sides(e, st);
+    if (!split) join_sides(e, st);
   } else {
   CVG_PAR(e);
   CVG_TRY(stage_x(e, x_real, B, fork_to(e, 1, st)));
@@ -1678,14 +1711,25 @@ int step_g(Engine& e, const float* x_real, int label, int B, const CvgNoise* nz,
   s.dpre = w.g_dout; s.sdpre = (long long)e.F * ld;
   s.coef_recon = e.cfg.lambda_recon / (Bg * (float)e.F);
   s.recon_acc = w.loss + L_RECON;
+  const unsigned seed_blocks = (unsigned)((e.F * ld + 255) / 256);
   if (e.mk.recording) {
     CVG_TRY(mk_push(e, mk::K_SEED, &s, sizeof(s), 2 * (int)(((long long)e.F * ld + mk::THREADS - 1) / mk::THREADS)));
+  } else if (split) {
+    const cudaStream_t sB = e.ms.s[1];
+    g_seed_kernel<<<dim3(seed_blocks, 1), 256, 0, st>>>(s);
+    CVG_LAUNCH_CHECK();
+    SeedArgs s1 = s;                                   // pass 1 alone: dx through the sigmoid
+    s1.out += (size_t)e.F * ld;
+    s1.dpre += (size_t)e.F * ld;
+    s1.prior_only = 1;
+    if (rng.lambda_nonzero) wait_for(e, sB, e.ms.s[0]);   // the classifier's share of dx
+    g_seed_kernel<<<dim3(seed_blocks, 1), 256, 0, sB>>>(s1);
+    CVG_LAUNCH_CHECK();
   } else {
-    g_seed_kernel<<<dim3((unsigned)((e.F * ld + 255) / 256), 2), 256, 0, st>>>(s);
+    g_seed_kernel<<<dim3(seed_blocks, 2), 256, 0, st>>>(s);
     CVG_LAUNCH_CHECK();
   }
 
-  const LinearP& g0 = lin(e, G, 0);
   BnNetBwd gb;
   gb.net = G; gb.npass = 2;
   gb.h = w.g_h; gb.dy = w.g_dy;
@@ -1697,8 +1741,7 @@ int step_g(Engine& e, const float* x_real, int label, int B, const CvgNoise* nz,
   gb.first_K = e.Z;
   gb.label_col = label_col_index(e, e.Z, label);
   gb.want_first_dx = true;
-  (void)g0;
-  CVG_TRY(bwd_bn_net(e, gb, B, Bg_bn, e.cfg.lambda_kl / Bg, local_bn, st));
+  const float kl_coef = e.cfg.lambda_kl / Bg;
 
   BnNetBwd eb;
   eb.net = E; eb.npass = 1;
@@ -1708,7 +1751,25 @@ int step_g(Engine& e, const float* x_real, int label, int B, const CvgNoise* nz,
   eb.first_K = e.F;
   eb.label_col = label_col_index(e, e.F, label);
   eb.want_first_dx = false;
-  CVG_TRY(bwd_bn_net(e, eb, B, Bg_bn, 0.f, local_bn, st));
+
+  if (split) {
+    const cudaStream_t sA = e.ms.s[0], sB = e.ms.s[1];
+    for (int l = 3; l >= 0; --l) {
+      wait_for(e, sA, st);                             // dY of layer l, pass 0 ...
+      wait_for(e, sA, sB);                             // ... and pass 1
+      CVG_TRY(bwd_bn_dx(e, gb, l, B, Bg_bn, kl_coef, local_bn, st, 0));
+      if (l > 0) CVG_TRY(bwd_bn_dx(e, gb, l, B, Bg_bn, kl_coef, local_bn, sB, 1));
+      CVG_TRY(bwd_bn_dw(e, gb, l, B, Bg_bn, local_bn, sA));
+    }
+    for (int l = 3; l >= 0; --l) {
+      const cudaStream_t sw = fork_to(e, 2, st);       // dY of layer l
+      CVG_TRY(bwd_bn_dx(e, eb, l, B, Bg_bn, 0.f, local_bn, st));
+      CVG_TRY(bwd_bn_dw(e, eb, l, B, Bg_bn, local_bn, sw));
+    }
+  } else {
+    CVG_TRY(bwd_bn_net(e, gb, B, Bg_bn, kl_coef, local_bn, st));
+    CVG_TRY(bwd_bn_net(e, eb, B, Bg_bn, 0.f, local_bn, st));
+  }
 
   CVG_TRY(finish_step(e, (1 << E) | (1 << G), 2, B, flags, loss_out, st));
   return prog.finish(st);
