@@ -437,6 +437,18 @@ static void add_job(FillArgs& a, void* out, const void* inj, int kind, int nfeat
   j.cstep = 0;
 }
 
+// the two dropout masks of the critic or the classifier, `npass` passes each
+static void add_masks(const Engine& e, FillArgs& f, int net, const CvgNoise* nz, int npass) {
+  const Workspace& w = e.ws;
+  if (net == CVG_NET_DISCRIMINATOR) {
+    add_job(f, w.d_m1, nz ? nz->d_mask1 : nullptr, 1, e.dh[0], npass, RS_DMASK1);
+    add_job(f, w.d_m2, nz ? nz->d_mask2 : nullptr, 1, e.dh[1], npass, RS_DMASK2);
+  } else {
+    add_job(f, w.c_m1, nz ? nz->c_mask1 : nullptr, 1, e.ch[0], npass, RS_CMASK1);
+    add_job(f, w.c_m2, nz ? nz->c_mask2 : nullptr, 1, e.ch[1], npass, RS_CMASK2);
+  }
+}
+
 static int emit_zero(Engine& e, void* p, size_t bytes, cudaStream_t st) {
   if (e.mk.recording) {
     mk::ZeroArgs a;
@@ -962,6 +974,23 @@ static int bwd_classifier(Engine& e, const float* xin, long long sxin, int npass
   return 0;
 }
 
+// The batch of one training step: B rows on this GPU, Bg over all GPUs (the losses are means over Bg), and the rows each
+// BatchNorm normalises over (Bg, or B with CVG_STEP_LOCAL_BN).
+struct StepDims {
+  int B;
+  bool local_bn;
+  float Bg, Bg_bn;
+};
+
+static StepDims step_dims(const Engine& e, int B, int flags) {
+  StepDims d;
+  d.B = B;
+  d.local_bn = flags & CVG_STEP_LOCAL_BN;
+  d.Bg = (float)B * (float)e.world;
+  d.Bg_bn = d.local_bn ? (float)B : d.Bg;
+  return d;
+}
+
 // BatchNorm MLP backward shared by generator (npass 2) and encoder (npass 1).
 //   top_dy      : dL/d(pre-activation of the last Linear) [Ntop][ld] per pass
 //   h[], dy[]   : the net's pre-BN activations and gradient scratch
@@ -975,6 +1004,7 @@ struct BnNetBwd {
   int first_K;             // its width
   int label_col;
   bool want_first_dx;      // generator: dL/dz_enc of pass 0 -> encoder head gradient
+  float kl_coef;           // with want_first_dx: weight of the KL term in that gradient
 };
 
 // dY operand of layer l: the gradient w.r.t. the output of its Linear
@@ -994,15 +1024,14 @@ static Operand bn_net_dy(const Engine& e, const BnNetBwd& b, int l) {
 
 // Input gradient of layer l: dY of layer l - 1 with its batch sums, or, at layer 0 with want_first_dx, the encoder head
 // gradient (pass 0 only).  Nothing at layer 0 otherwise.  only_pass >= 0: that pass alone, in a grid of one pass slot.
-static int bwd_bn_dx(Engine& e, const BnNetBwd& b, int l, int M, float Bg_bn, float kl_coef, bool local_bn, cudaStream_t st,
-                     int only_pass = -1) {
+static int bwd_bn_dx(Engine& e, const BnNetBwd& b, int l, const StepDims& d, cudaStream_t st, int only_pass = -1) {
   const Workspace& w = e.ws;
   const size_t ld = w.ld;
   const int net = b.net;
   const LinearP& p = lin(e, net, l);
   if (l > 0) {
     const LinearP& pp = lin(e, net, l - 1);
-    GemmArgs g = base_args(e, M, Bg_bn, b.npass);
+    GemmArgs g = base_args(e, d.B, d.Bg_bn, b.npass);
     g.only_pass = only_pass;
     g.R = p.out;
     g.N = p.in;
@@ -1017,10 +1046,10 @@ static int bwd_bn_dx(Engine& e, const BnNetBwd& b, int l, int M, float Bg_bn, fl
     g.sY = (long long)pp.out * ld;
     g.ostats = bst_of(e, net, l - 1);
     g.sostats = 2 * STAT_C;
-    return launch_mn_stats(e, false, g, b.npass, local_bn, st);
+    return launch_mn_stats(e, false, g, b.npass, d.local_bn, st);
   }
   if (!b.want_first_dx) return 0;
-  GemmArgs g = base_args(e, M, Bg_bn, b.npass);
+  GemmArgs g = base_args(e, d.B, d.Bg_bn, b.npass);
   g.only_pass = 0;
   g.R = p.out;
   g.N = e.Z;
@@ -1031,16 +1060,16 @@ static int bwd_bn_dx(Engine& e, const BnNetBwd& b, int l, int M, float Bg_bn, fl
   g.mu = w.e_ml;
   g.lv = w.e_ml + (size_t)e.Z * ld;
   g.eps = e.mk.recording ? w.z_eps : w.z;
-  g.kl_coef = kl_coef;
+  g.kl_coef = b.kl_coef;
   g.Y = w.e_dml;
   return launch_mn(e, false, g, st);
 }
 
 // dW, db and the BatchNorm affine gradients of layer l, all passes in one launch
-static int bwd_bn_dw(Engine& e, const BnNetBwd& b, int l, int M, float Bg_bn, bool local_bn, cudaStream_t st) {
+static int bwd_bn_dw(Engine& e, const BnNetBwd& b, int l, const StepDims& sd, cudaStream_t st) {
   const int net = b.net;
   const LinearP& p = lin(e, net, l);
-  DwArgs d = base_dw(e, M, Bg_bn, b.npass);
+  DwArgs d = base_dw(e, sd.B, sd.Bg_bn, b.npass);
   d.N = p.out;
   d.p = bn_net_dy(e, b, l);
   if (l == 0) {
@@ -1064,19 +1093,55 @@ static int bwd_bn_dw(Engine& e, const BnNetBwd& b, int l, int M, float Bg_bn, bo
     d.dbeta = e.G(net, p.beta);
     // with global BatchNorm the sums are already global: only rank 0 contributes them before the
     // gradient all-reduce (sum).  With local BatchNorm every rank adds its own.
-    d.add_affine = (e.world <= 1 || local_bn || e.rank == 0) ? 1 : 0;
+    d.add_affine = (e.world <= 1 || sd.local_bn || e.rank == 0) ? 1 : 0;
   }
   return launch_dw(e, d, st);
 }
 
-static int bwd_bn_net(Engine& e, const BnNetBwd& b, int M, float Bg_bn, float kl_coef, bool local_bn, cudaStream_t st) {
+static int bwd_bn_net(Engine& e, const BnNetBwd& b, const StepDims& d, cudaStream_t st) {
   for (int l = 3; l >= 0; --l) {
     // dX first: it produces the batch sums the next layer's kernels need
-    CVG_TRY(bwd_bn_dx(e, b, l, M, Bg_bn, kl_coef, local_bn, st));
+    CVG_TRY(bwd_bn_dx(e, b, l, d, st));
     if (l > 0 || b.want_first_dx) CVG_PAR(e);     // beside the input-gradient op just emitted: both read dY of layer l
-    CVG_TRY(bwd_bn_dw(e, b, l, M, Bg_bn, local_bn, fork_to(e, 0, st)));
+    CVG_TRY(bwd_bn_dw(e, b, l, d, fork_to(e, 0, st)));
   }
   return 0;
+}
+
+// The generator's backward over `npass` passes.  first_kind: how its first Linear reads z, OP_REPARAM where pass 0
+// computes z_enc = mu + eps * std in the operand load, OP_PLAIN where z is read as stored.  want_first_dx: the pass-0 input
+// gradient goes on to the encoder head (dL/dmu, dL/dlogvar, with the KL term).
+static BnNetBwd gen_bwd(const Engine& e, const StepDims& d, int npass, int first_kind, int label, bool want_first_dx) {
+  const Workspace& w = e.ws;
+  BnNetBwd b;
+  b.net = CVG_NET_GENERATOR; b.npass = npass;
+  b.h = w.g_h; b.dy = w.g_dy;
+  b.top_dy = w.g_dout; b.s_top = (long long)e.F * w.ld;
+  b.first_in.kind = first_kind; b.first_in.rows = e.Z;
+  b.first_in.p = w.z; b.first_in.sp = (long long)e.Z * w.ld;
+  if (want_first_dx) {   // pass 0 is z_enc
+    b.first_in.mu = w.e_ml; b.first_in.lv = w.e_ml + (size_t)e.Z * w.ld; b.first_in.eps = w.z;
+    b.first_in.reparam_pass = 0;
+  }
+  b.first_K = e.Z;
+  b.label_col = label_col_index(e, e.Z, label);
+  b.want_first_dx = want_first_dx;
+  b.kl_coef = want_first_dx ? e.cfg.lambda_kl / d.Bg : 0.f;
+  return b;
+}
+
+static BnNetBwd enc_bwd(const Engine& e, int label) {
+  const Workspace& w = e.ws;
+  BnNetBwd b;
+  b.net = CVG_NET_ENCODER; b.npass = 1;
+  b.h = w.e_h; b.dy = w.e_dy;
+  b.top_dy = w.e_dml; b.s_top = 0;
+  b.first_in.kind = OP_PLAIN; b.first_in.rows = e.F; b.first_in.p = w.xT;
+  b.first_K = e.F;
+  b.label_col = label_col_index(e, e.F, label);
+  b.want_first_dx = false;
+  b.kl_coef = 0.f;
+  return b;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1275,10 +1340,81 @@ static int prep_net(Engine& e, int net, bool fwd, bool dx, bool first_dx) {
   return 0;
 }
 
-static int emit_ce(Engine& e, const CeArgs& c, int B, int npass, cudaStream_t st) {
-  if (e.mk.recording) return mk_push(e, mk::K_CE, &c, sizeof(c), npass * ((B + mk::THREADS - 1) / mk::THREADS));
-  ce_kernel<<<dim3((B + 127) / 128, npass), 128, 0, st>>>(c);
+// Cross-entropy of the classifier's logits against the shared `label`, or against per-row `labels` when given.  The
+// gradient is scaled by 1 / Bg, and also by ctl->lambda_class when `ctl` is set (read on the device).
+static CeArgs ce_args(const Engine& e, const StepDims& d, int npass, int label, const long long* labels, const StepCtl* ctl) {
+  const Workspace& w = e.ws;
+  CeArgs c;
+  c.M = d.B; c.ld = w.ld; c.K = e.K; c.npass = npass; c.label = label; c.labels = labels;
+  c.logits = w.c_logit; c.sl = (long long)e.K * w.ld;
+  c.dlogits = w.c_dlogit; c.sd = (long long)e.K * w.ld;
+  c.coef = 1.0f / d.Bg;
+  c.ctl = ctl;
+  c.loss = w.loss + L_CE0;
+  return c;
+}
+
+static int emit_ce(Engine& e, const CeArgs& c, cudaStream_t st) {
+  if (e.mk.recording) return mk_push(e, mk::K_CE, &c, sizeof(c), c.npass * ((c.M + mk::THREADS - 1) / mk::THREADS));
+  ce_kernel<<<dim3((c.M + 127) / 128, c.npass), 128, 0, st>>>(c);
   CVG_LAUNCH_CHECK();
+  return 0;
+}
+
+// Generator output gradients: the reconstruction MSE (weight coef_recon) on pass 0, ws.dx on pass 1, through the sigmoid
+static SeedArgs seed_args(const Engine& e, int B, float coef_recon) {
+  const Workspace& w = e.ws;
+  SeedArgs s;
+  s.M = B; s.ld = w.ld; s.F = e.F;
+  s.out = w.g_out; s.sout = (long long)e.F * w.ld;
+  s.x = w.xT; s.dx = w.dx;
+  s.dpre = w.g_dout; s.sdpre = (long long)e.F * w.ld;
+  s.coef_recon = coef_recon;
+  s.recon_acc = w.loss + L_RECON;
+  return s;
+}
+
+// `npass` passes of the seed, from s.out on
+static int launch_seed(Engine& e, const SeedArgs& s, int npass, cudaStream_t st) {
+  const long long n = (long long)e.F * e.ws.ld;
+  if (e.mk.recording) return mk_push(e, mk::K_SEED, &s, sizeof(s), npass * (int)((n + mk::THREADS - 1) / mk::THREADS));
+  g_seed_kernel<<<dim3((unsigned)((n + 255) / 256), npass), 256, 0, st>>>(s);
+  CVG_LAUNCH_CHECK();
+  return 0;
+}
+
+// ------------------------------------------------------------------------------------------------
+// head of the D and C steps: `net` is the critic or the classifier, which scores the real batch (pass 0) and x_fake = G(z)
+// (pass 1).  Returns in *sx the offset from the staged batch to x_fake.
+// ------------------------------------------------------------------------------------------------
+static int dc_head(Engine& e, int net, const float* x_real, int label, const StepDims& d, const CvgNoise* nz,
+                   const StepRng& rng, cudaStream_t st, long long* sx) {
+  const Workspace& w = e.ws;
+  const bool critic = net == CVG_NET_DISCRIMINATOR;
+  if (rng.set) CVG_PAR(e);
+  CVG_TRY(emit_zero(e, w.acc, w.acc_bytes, st));
+  if (critic) {
+    CVG_PAR(e);
+    CVG_TRY(emit_zero(e, w.sn_G, sizeof(float) * 2 * e.lay[net].n_param, st));
+  }
+  CVG_TRY(prep_net(e, CVG_NET_GENERATOR, true, false, false));
+  CVG_TRY(prep_net(e, net, true, true, false));
+  FillArgs f;
+  fill_args(e, f, rng, d.B);
+  if (!e.hoist_x) add_job(f, w.z, nz ? nz->z : nullptr, 0, e.Z, 1, RS_Z);
+  add_masks(e, f, net, nz, 2);
+  CVG_PAR(e);
+  CVG_TRY(launch_fill(e, f, st));
+  CVG_PAR(e);
+  CVG_TRY(stage_x(e, x_real, d.B, fork_to(e, 1, st)));
+  if (critic) {
+    CVG_PAR(e);                           // the power iterations only touch the critic's weights and u / v: first phase
+    CVG_TRY(launch_sn(e, 2, true, fork_to(e, 0, st)));   // D(real) then D(fake): two consecutive power iterations
+  }
+  // G(z) under no_grad, still in train mode: batch stats, running stats updated (cvae_gan.py:113-115)
+  if (!e.hoist_x) CVG_TRY(fwd_generator(e, 1, true, false, label, d.B, d.Bg_bn, d.local_bn, st));
+  join_sides(e, st);
+  *sx = (e.hoist_x ? e.hoist_x : w.g_out) - w.xT;  // pass 0 reads xT, pass 1 reads G(z)
   return 0;
 }
 
@@ -1291,32 +1427,11 @@ int step_d(Engine& e, const float* x_real, int label, int B, const CvgNoise* nz,
   ProgramScope prog(e);
   CVG_TRY(begin_step(e, rng, false, st));
   const Workspace& w = e.ws;
-  const bool local_bn = flags & CVG_STEP_LOCAL_BN;
-  const float Bg = (float)B * (float)e.world;
-  const float Bg_bn = local_bn ? (float)B : Bg;
+  const StepDims d = step_dims(e, B, flags);
   const int D = CVG_NET_DISCRIMINATOR;
-  if (rng.set) CVG_PAR(e);
-  CVG_TRY(emit_zero(e, w.acc, w.acc_bytes, st));
-  CVG_PAR(e);
-  CVG_TRY(emit_zero(e, w.sn_G, sizeof(float) * 2 * e.lay[D].n_param, st));
-  CVG_TRY(prep_net(e, CVG_NET_GENERATOR, true, false, false));
-  CVG_TRY(prep_net(e, D, true, true, false));
-  FillArgs f;
-  fill_args(e, f, rng, B);
-  if (!e.hoist_x) add_job(f, w.z, nz ? nz->z : nullptr, 0, e.Z, 1, RS_Z);
-  add_job(f, w.d_m1, nz ? nz->d_mask1 : nullptr, 1, e.dh[0], 2, RS_DMASK1);
-  add_job(f, w.d_m2, nz ? nz->d_mask2 : nullptr, 1, e.dh[1], 2, RS_DMASK2);
-  CVG_PAR(e);
-  CVG_TRY(launch_fill(e, f, st));
-  CVG_PAR(e);
-  CVG_TRY(stage_x(e, x_real, B, fork_to(e, 1, st)));
-  CVG_PAR(e);                           // the power iterations only touch the critic's weights and u / v: first phase
-  CVG_TRY(launch_sn(e, 2, true, fork_to(e, 0, st)));   // D(real) then D(fake): two consecutive power iterations
-  // G(z) under no_grad, still in train mode: batch stats, running stats updated (cvae_gan.py:113-115)
-  if (!e.hoist_x) CVG_TRY(fwd_generator(e, 1, true, false, label, B, Bg_bn, local_bn, st));
-  join_sides(e, st);
-  const long long sx = (e.hoist_x ? e.hoist_x : w.g_out) - w.xT;  // pass 0 reads xT, pass 1 reads G(z)
-  const float seedv[2] = {-1.0f / Bg, 1.0f / Bg};   // d_loss = -mean D(real) + mean D(fake)
+  long long sx;
+  CVG_TRY(dc_head(e, D, x_real, label, d, nz, rng, st, &sx));
+  const float seedv[2] = {-1.0f / d.Bg, 1.0f / d.Bg};   // d_loss = -mean D(real) + mean D(fake)
   if (chain_usable(e, D)) {
     CVG_TRY(launch_critic_chain(e, sx, label, B, seedv, st));
     CVG_TRY(bwd_critic(e, w.xT, sx, 2, label, B, seedv, true, false, st, true));
@@ -1368,40 +1483,16 @@ int step_c(Engine& e, const float* x_real, int label, int B, const CvgNoise* nz,
   ProgramScope prog(e);
   CVG_TRY(begin_step(e, rng, false, st));
   const Workspace& w = e.ws;
-  const size_t ld = w.ld;
-  const bool local_bn = flags & CVG_STEP_LOCAL_BN;
-  const float Bg = (float)B * (float)e.world;
-  const float Bg_bn = local_bn ? (float)B : Bg;
+  const StepDims d = step_dims(e, B, flags);
   const int C = CVG_NET_CLASSIFIER;
-  if (rng.set) CVG_PAR(e);
-  CVG_TRY(emit_zero(e, w.acc, w.acc_bytes, st));
-  CVG_TRY(prep_net(e, CVG_NET_GENERATOR, true, false, false));
-  CVG_TRY(prep_net(e, C, true, true, false));
-  FillArgs f;
-  fill_args(e, f, rng, B);
-  if (!e.hoist_x) add_job(f, w.z, nz ? nz->z : nullptr, 0, e.Z, 1, RS_Z);
-  add_job(f, w.c_m1, nz ? nz->c_mask1 : nullptr, 1, e.ch[0], 2, RS_CMASK1);
-  add_job(f, w.c_m2, nz ? nz->c_mask2 : nullptr, 1, e.ch[1], 2, RS_CMASK2);
-  CVG_PAR(e);
-  CVG_TRY(launch_fill(e, f, st));
-  CVG_PAR(e);
-  CVG_TRY(stage_x(e, x_real, B, fork_to(e, 1, st)));
-  if (!e.hoist_x) CVG_TRY(fwd_generator(e, 1, true, false, label, B, Bg_bn, local_bn, st));
-  join_sides(e, st);
-  const long long sx = (e.hoist_x ? e.hoist_x : w.g_out) - w.xT;
+  long long sx;
+  CVG_TRY(dc_head(e, C, x_real, label, d, nz, rng, st, &sx));
   if (chain_usable(e, C)) {
-    CVG_TRY(launch_classifier_chain(e, sx, label, B, 1.0f / Bg, st));
+    CVG_TRY(launch_classifier_chain(e, sx, label, B, 1.0f / d.Bg, st));
     CVG_TRY(bwd_classifier(e, w.xT, sx, 2, B, true, false, false, st, nullptr, true));
   } else {
     CVG_TRY(fwd_classifier(e, w.xT, sx, 2, true, B, st));
-    CeArgs c;
-    c.M = B; c.ld = w.ld; c.K = e.K; c.npass = 2; c.label = label;
-    c.logits = w.c_logit; c.sl = (long long)e.K * ld;
-    c.dlogits = w.c_dlogit; c.sd = (long long)e.K * ld;
-    c.coef = 1.0f / Bg;
-    c.ctl = nullptr;
-    c.loss = w.loss + L_CE0;
-    CVG_TRY(emit_ce(e, c, B, 2, st));
+    CVG_TRY(emit_ce(e, ce_args(e, d, 2, label, nullptr, nullptr), st));
     CVG_TRY(bwd_classifier(e, w.xT, sx, 2, B, true, false, false, st));
   }
   CVG_TRY(finish_step(e, 1 << C, 1, B, flags, loss_out, st));
@@ -1419,29 +1510,20 @@ int step_classifier(Engine& e, const float* x, const long long* labels, int B, c
   ProgramScope prog(e);
   CVG_TRY(begin_step(e, rng, false, st));
   const Workspace& w = e.ws;
-  const size_t ld = w.ld;
+  const StepDims d = step_dims(e, B, flags);
   const int C = CVG_NET_CLASSIFIER;
-  const float Bg = (float)B * (float)e.world;
   if (rng.set) CVG_PAR(e);
   CVG_TRY(emit_zero(e, w.acc, w.acc_bytes, st));
   CVG_TRY(prep_net(e, C, true, true, false));
   FillArgs f;
   fill_args(e, f, rng, B);
-  add_job(f, w.c_m1, nz ? nz->c_mask1 : nullptr, 1, e.ch[0], 1, RS_CMASK1);
-  add_job(f, w.c_m2, nz ? nz->c_mask2 : nullptr, 1, e.ch[1], 1, RS_CMASK2);
+  add_masks(e, f, C, nz, 1);
   CVG_PAR(e);
   CVG_TRY(launch_fill(e, f, st));
   CVG_PAR(e);
   CVG_TRY(stage_x(e, x, B, st));
   CVG_TRY(fwd_classifier(e, w.xT, 0, 1, true, B, st));
-  CeArgs c;
-  c.M = B; c.ld = w.ld; c.K = e.K; c.npass = 1; c.label = 0; c.labels = labels;
-  c.logits = w.c_logit; c.sl = (long long)e.K * ld;
-  c.dlogits = w.c_dlogit; c.sd = (long long)e.K * ld;
-  c.coef = 1.0f / Bg;
-  c.ctl = nullptr;
-  c.loss = w.loss + L_CE0;
-  CVG_TRY(emit_ce(e, c, B, 1, st));
+  CVG_TRY(emit_ce(e, ce_args(e, d, 1, 0, labels, nullptr), st));
   CVG_TRY(bwd_classifier(e, w.xT, 0, 1, B, true, false, false, st));
   CVG_TRY(finish_step(e, 1 << C, 1, B, flags, loss_out, st, &ov));
   return prog.finish(st);
@@ -1450,6 +1532,20 @@ int step_classifier(Engine& e, const float* x, const long long* labels, int B, c
 // ------------------------------------------------------------------------------------------------
 // step E+G (cvae_gan.py:160-216)
 // ------------------------------------------------------------------------------------------------
+// The critic's and the classifier's terms of a generator step, as one chain each: D(x_fake) forward and backward to ws.dx
+// on st; C(x_fake) forward and loss on sc (the class loss is reported even while its weight is 0, cgan.py:162,181) and,
+// with lambda_class != 0, its backward added into ws.dx after the critic's.  sc == st runs both as one chain.
+static int score_fake(Engine& e, const float* x_fake, int label, const StepDims& d, bool lambda_nonzero, cudaStream_t st,
+                      cudaStream_t sc) {
+  const float seedv[2] = {-e.cfg.lambda_adv / d.Bg, 0.f};   // adv = -mean D(x_fake) (cvae_gan.py:189)
+  CVG_TRY(fwd_critic(e, x_fake, 0, 1, label, d.B, e.ws.loss + L_DFAKE, st));
+  CVG_TRY(fwd_classifier(e, x_fake, 0, 1, true, d.B, sc));
+  CVG_TRY(emit_ce(e, ce_args(e, d, 1, label, nullptr, e.ws.ctl), sc));
+  CVG_TRY(bwd_critic(e, x_fake, 0, 1, label, d.B, seedv, false, true, st));
+  if (lambda_nonzero) CVG_TRY(bwd_classifier(e, x_fake, 0, 1, d.B, false, true, true, sc, st));
+  return 0;
+}
+
 // ------------------------------------------------------------------------------------------------
 // Sibling trainer CGAN (SURVEY 8 f4), generator step (/root/reference/src/cgan.py:138-178): x_fake = G(z_prior, onehot)
 // only - no encoder, no reconstruction / KL terms, no real batch -, total = lambda_adv * (-mean D(x_fake)) +
@@ -1462,62 +1558,26 @@ static int step_g_prior(Engine& e, int label, int B, const CvgNoise* nz, const S
   if (e.mk.recording || mk_usable(e)) CVG_FAIL("the CGAN generator step runs on the stand-alone executor only (unset CVG_TRAIN_MODE)");
   CVG_TRY(begin_step(e, rng, true, st));
   const Workspace& w = e.ws;
-  const size_t ld = w.ld;
-  const bool local_bn = flags & CVG_STEP_LOCAL_BN;
-  const float Bg = (float)B * (float)e.world;
-  const float Bg_bn = local_bn ? (float)B : Bg;
+  const StepDims d = step_dims(e, B, flags);
   const int G = CVG_NET_GENERATOR;
   CVG_TRY(emit_zero(e, w.acc, w.acc_bytes, st));
   FillArgs f;
   fill_args(e, f, rng, B);
   add_job(f, w.z, nz ? nz->z : nullptr, 0, e.Z, 1, RS_Z);
-  add_job(f, w.d_m1, nz ? nz->d_mask1 : nullptr, 1, e.dh[0], 1, RS_DMASK1);
-  add_job(f, w.d_m2, nz ? nz->d_mask2 : nullptr, 1, e.dh[1], 1, RS_DMASK2);
-  add_job(f, w.c_m1, nz ? nz->c_mask1 : nullptr, 1, e.ch[0], 1, RS_CMASK1);
-  add_job(f, w.c_m2, nz ? nz->c_mask2 : nullptr, 1, e.ch[1], 1, RS_CMASK2);
+  add_masks(e, f, CVG_NET_DISCRIMINATOR, nz, 1);
+  add_masks(e, f, CVG_NET_CLASSIFIER, nz, 1);
   CVG_TRY(launch_fill(e, f, st));
   join_sides(e, st);                                     // the previous step's Adam (visit: side stream 0)
   CVG_TRY(launch_sn(e, 1, true, fork_to(e, 0, st)));
-  CVG_TRY(fwd_generator(e, 1, true, false, label, B, Bg_bn, local_bn, st));
+  CVG_TRY(fwd_generator(e, 1, true, false, label, B, d.Bg_bn, d.local_bn, st));
   join_sides(e, st);
-  const float* x_fake = w.g_out;
   const cudaStream_t sc = fork_to(e, 1, st);
-  CVG_TRY(fwd_critic(e, x_fake, 0, 1, label, B, w.loss + L_DFAKE, st));
-  {                                                      // the class loss is reported even while its weight is 0 (cgan.py:162,181)
-    CVG_TRY(fwd_classifier(e, x_fake, 0, 1, true, B, sc));
-    CeArgs c;
-    c.M = B; c.ld = w.ld; c.K = e.K; c.npass = 1; c.label = label;
-    c.logits = w.c_logit; c.sl = (long long)e.K * ld;
-    c.dlogits = w.c_dlogit; c.sd = (long long)e.K * ld;
-    c.coef = 1.0f / Bg;       // times ctl->lambda_class, read on the device
-    c.ctl = w.ctl;
-    c.loss = w.loss + L_CE0;
-    CVG_TRY(emit_ce(e, c, B, 1, sc));
-  }
-  const float seedv[2] = {-e.cfg.lambda_adv / Bg, 0.f};
-  CVG_TRY(bwd_critic(e, x_fake, 0, 1, label, B, seedv, false, true, st));
-  if (rng.lambda_nonzero) CVG_TRY(bwd_classifier(e, x_fake, 0, 1, B, false, true, true, sc, st));
+  CVG_TRY(score_fake(e, w.g_out, label, d, rng.lambda_nonzero, st, sc));
   join_sides(e, st);
-  SeedArgs s;
-  s.M = B; s.ld = w.ld; s.F = e.F;
-  s.out = w.g_out; s.sout = (long long)e.F * ld;
-  s.x = w.xT; s.dx = w.dx;
-  s.dpre = w.g_dout; s.sdpre = (long long)e.F * ld;
-  s.coef_recon = 0.f;
-  s.recon_acc = w.loss + L_RECON;
+  SeedArgs s = seed_args(e, B, 0.f);
   s.prior_only = 1;
-  g_seed_kernel<<<dim3((unsigned)((e.F * ld + 255) / 256), 1), 256, 0, st>>>(s);
-  CVG_LAUNCH_CHECK();
-  BnNetBwd gb;
-  gb.net = G; gb.npass = 1;
-  gb.h = w.g_h; gb.dy = w.g_dy;
-  gb.top_dy = w.g_dout; gb.s_top = (long long)e.F * ld;
-  gb.first_in.kind = OP_PLAIN; gb.first_in.rows = e.Z;
-  gb.first_in.p = w.z; gb.first_in.sp = (long long)e.Z * ld;
-  gb.first_K = e.Z;
-  gb.label_col = label_col_index(e, e.Z, label);
-  gb.want_first_dx = false;
-  CVG_TRY(bwd_bn_net(e, gb, B, Bg_bn, 0.f, local_bn, st));
+  CVG_TRY(launch_seed(e, s, 1, st));
+  CVG_TRY(bwd_bn_net(e, gen_bwd(e, d, 1, OP_PLAIN, label, false), d, st));
   return finish_step(e, 1 << G, 2, B, flags, loss_out, st);
 }
 
@@ -1535,67 +1595,138 @@ static int step_g_cvae(Engine& e, const float* x_real, int label, int B, const C
   if (e.mk.recording || mk_usable(e)) CVG_FAIL("the CVAE encoder/generator step runs on the stand-alone executor only (unset CVG_TRAIN_MODE)");
   CVG_TRY(begin_step(e, rng, true, st));
   const Workspace& w = e.ws;
-  const size_t ld = w.ld;
-  const bool local_bn = flags & CVG_STEP_LOCAL_BN;
-  const float Bg = (float)B * (float)e.world;
-  const float Bg_bn = local_bn ? (float)B : Bg;
+  const StepDims d = step_dims(e, B, flags);
   const int E = CVG_NET_ENCODER, G = CVG_NET_GENERATOR;
   CVG_TRY(emit_zero(e, w.acc, w.acc_bytes, st));
   FillArgs f;
   fill_args(e, f, rng, B);
   add_job(f, w.z, nz ? nz->eps : nullptr, 0, e.Z, 1, RS_EPS);     // eps in slot 0: reparameterisation fused into G's first operand load
-  add_job(f, w.c_m1, nz ? nz->c_mask1 : nullptr, 1, e.ch[0], 1, RS_CMASK1);
-  add_job(f, w.c_m2, nz ? nz->c_mask2 : nullptr, 1, e.ch[1], 1, RS_CMASK2);
+  add_masks(e, f, CVG_NET_CLASSIFIER, nz, 1);
   CVG_TRY(launch_fill(e, f, st));
   join_sides(e, st);                                     // the previous step's Adam (visit: side stream 0)
   CVG_TRY(stage_x(e, x_real, B, st));
-  CVG_TRY(fwd_encoder(e, true, label, B, Bg_bn, local_bn, st));
-  CVG_TRY(fwd_generator(e, 1, true, true, label, B, Bg_bn, local_bn, st));
+  CVG_TRY(fwd_encoder(e, true, label, B, d.Bg_bn, d.local_bn, st));
+  CVG_TRY(fwd_generator(e, 1, true, true, label, B, d.Bg_bn, d.local_bn, st));
   const float* x_recon = w.g_out;
-  {                                                      // the class loss is reported even while its weight is 0 (cvae.py:141-142,162)
-    CVG_TRY(fwd_classifier(e, x_recon, 0, 1, true, B, st));
-    CeArgs c;
-    c.M = B; c.ld = w.ld; c.K = e.K; c.npass = 1; c.label = label;
-    c.logits = w.c_logit; c.sl = (long long)e.K * ld;
-    c.dlogits = w.c_dlogit; c.sd = (long long)e.K * ld;
-    c.coef = 1.0f / Bg;       // times ctl->lambda_class, read on the device
-    c.ctl = w.ctl;
-    c.loss = w.loss + L_CE0;
-    CVG_TRY(emit_ce(e, c, B, 1, st));
-  }
+  // the class loss is reported even while its weight is 0 (cvae.py:141-142,162)
+  CVG_TRY(fwd_classifier(e, x_recon, 0, 1, true, B, st));
+  CVG_TRY(emit_ce(e, ce_args(e, d, 1, label, nullptr, w.ctl), st));
   if (rng.lambda_nonzero) CVG_TRY(bwd_classifier(e, x_recon, 0, 1, B, false, true, false, st));   // -> ws.dx
-  SeedArgs s;
-  s.M = B; s.ld = w.ld; s.F = e.F;
-  s.out = w.g_out; s.sout = (long long)e.F * ld;
-  s.x = w.xT; s.dx = w.dx;
-  s.dpre = w.g_dout; s.sdpre = (long long)e.F * ld;
-  s.coef_recon = e.cfg.lambda_recon / (Bg * (float)e.F);
-  s.recon_acc = w.loss + L_RECON;
+  SeedArgs s = seed_args(e, B, e.cfg.lambda_recon / (d.Bg * (float)e.F));
   s.add_dx = rng.lambda_nonzero ? 1 : 0;
-  g_seed_kernel<<<dim3((unsigned)((e.F * ld + 255) / 256), 1), 256, 0, st>>>(s);
-  CVG_LAUNCH_CHECK();
-  BnNetBwd gb;
-  gb.net = G; gb.npass = 1;
-  gb.h = w.g_h; gb.dy = w.g_dy;
-  gb.top_dy = w.g_dout; gb.s_top = (long long)e.F * ld;
-  gb.first_in.kind = OP_REPARAM; gb.first_in.rows = e.Z;
-  gb.first_in.p = w.z; gb.first_in.sp = (long long)e.Z * ld;
-  gb.first_in.mu = w.e_ml; gb.first_in.lv = w.e_ml + (size_t)e.Z * ld; gb.first_in.eps = w.z;
-  gb.first_in.reparam_pass = 0;
-  gb.first_K = e.Z;
-  gb.label_col = label_col_index(e, e.Z, label);
-  gb.want_first_dx = true;
-  CVG_TRY(bwd_bn_net(e, gb, B, Bg_bn, e.cfg.lambda_kl / Bg, local_bn, st));
-  BnNetBwd eb;
-  eb.net = E; eb.npass = 1;
-  eb.h = w.e_h; eb.dy = w.e_dy;
-  eb.top_dy = w.e_dml; eb.s_top = 0;
-  eb.first_in.kind = OP_PLAIN; eb.first_in.rows = e.F; eb.first_in.p = w.xT;
-  eb.first_K = e.F;
-  eb.label_col = label_col_index(e, e.F, label);
-  eb.want_first_dx = false;
-  CVG_TRY(bwd_bn_net(e, eb, B, Bg_bn, 0.f, local_bn, st));
+  CVG_TRY(launch_seed(e, s, 1, st));
+  CVG_TRY(bwd_bn_net(e, gen_bwd(e, d, 1, OP_REPARAM, label, true), d, st));
+  CVG_TRY(bwd_bn_net(e, enc_bwd(e, label), d, st));
   return finish_step(e, (1 << E) | (1 << G), 2, B, flags, loss_out, st);
+}
+
+// How the E/G step enqueues its work.  With the stand-alone kernels and the side streams on, the forward runs as three
+// chains side by side, and the backward as one chain (THREE) or with one generator chain per pass (SPLIT).  ONE_CHAIN runs
+// one chain with a few branches beside it: in the step-program recorder, with the side streams off, and on several GPUs
+// whose BatchNorm exchange is not folded into the kernels.
+enum class EgSchedule { ONE_CHAIN, THREE, SPLIT };
+
+// SPLIT only where no BatchNorm sums are exchanged: a folded exchange of one pass cannot yet be told from the other pass's.
+static EgSchedule eg_schedule(const Engine& e, bool local_bn) {
+  const bool three = !e.mk.recording && e.ms.on && (e.world <= 1 || local_bn || fold_stats(e, local_bn));
+  const bool split = three && e.eg_split && (e.world <= 1 || local_bn);
+  return split ? EgSchedule::SPLIT : three ? EgSchedule::THREE : EgSchedule::ONE_CHAIN;
+}
+
+// Forward of THREE and SPLIT (data parallel: with the folded exchange, one channel per chain): x_fake = G(z_prior) does not
+// depend on the encoder, and the critic / classifier terms only on x_fake.
+//   caller's stream : E(x), G(z_enc)
+//   side 1          : batch staging, G(z_prior), then D(x_fake) forward and backward to x_fake
+//   side 0          : power iteration, then C(x_fake) forward, loss and backward to x_fake (after D's: both add to ws.dx)
+// With lambda_class = 0 the classifier's forward and loss are skipped, so these schedules report a class loss of 0 where
+// ONE_CHAIN (and the reference) report the cross-entropy.
+static int eg_fwd_three(Engine& e, const float* x_real, int label, const StepDims& d, bool lambda_nonzero, cudaStream_t st) {
+  const Workspace& w = e.ws;
+  const float* x_fake = w.g_out + (size_t)e.F * w.ld;
+  const float seedv[2] = {-e.cfg.lambda_adv / d.Bg, 0.f};   // adv = -mean D(x_fake) (cvae_gan.py:189)
+  const cudaStream_t sA = fork_to(e, 0, st), sB = fork_to(e, 1, st);
+  CVG_TRY(launch_sn(e, 1, true, sA));
+  CVG_TRY(stage_x(e, x_real, d.B, sB));
+  wait_for(e, st, sB);                                            // the encoder reads the staged batch
+  GenSplit prior;
+  prior.only_pass = 1; prior.channel = 1; prior.rec = e.ms.layer;
+  CVG_TRY(fwd_generator(e, 2, true, false, label, d.B, d.Bg_bn, d.local_bn, sB, nullptr, &prior));
+  wait_for(e, sB, sA);                                            // sigma of the critic's layers (all side 0 holds so far)
+  if (lambda_nonzero) {
+    wait_for(e, sA, sB);                                          // x_fake
+    CVG_TRY(fwd_classifier(e, x_fake, 0, 1, true, d.B, sA));
+    CVG_TRY(emit_ce(e, ce_args(e, d, 1, label, nullptr, w.ctl), sA));
+  }
+  CVG_TRY(fwd_critic(e, x_fake, 0, 1, label, d.B, w.loss + L_DFAKE, sB));
+  CVG_TRY(bwd_critic(e, x_fake, 0, 1, label, d.B, seedv, false, true, sB));
+  if (lambda_nonzero) CVG_TRY(bwd_classifier(e, x_fake, 0, 1, d.B, false, true, true, sA, sB));
+  CVG_TRY(fwd_encoder(e, true, label, d.B, d.Bg_bn, d.local_bn, st));
+  GenSplit enc;
+  enc.only_pass = 0; enc.channel = 0; enc.wait = e.ms.layer;
+  return fwd_generator(e, 2, true, true, label, d.B, d.Bg_bn, d.local_bn, st, nullptr, &enc);
+}
+
+// Forward of ONE_CHAIN: E -> (mu, logvar); G on z_enc (pass 0) and z_prior (pass 1); D and C on x_fake
+static int eg_fwd_one(Engine& e, const float* x_real, int label, const StepDims& d, bool lambda_nonzero, cudaStream_t st) {
+  const Workspace& w = e.ws;
+  CVG_PAR(e);
+  CVG_TRY(stage_x(e, x_real, d.B, fork_to(e, 1, st)));
+  CVG_PAR(e);
+  CVG_TRY(launch_sn(e, 1, true, fork_to(e, 0, st)));   // critic power iteration: independent of everything before D(x_fake)
+  join_sides(e, st, 1);
+  CVG_TRY(fwd_encoder(e, true, label, d.B, d.Bg_bn, d.local_bn, st));
+  if (e.mk.recording) {
+    mk::ReparamArgs ra;
+    ra.mu = w.e_ml; ra.lv = w.e_ml + (size_t)e.Z * w.ld; ra.eps = w.z_eps; ra.out = w.z; ra.M = d.B; ra.ld = w.ld; ra.Z = e.Z;
+    CVG_TRY(mk_push(e, mk::K_REPARAM, &ra, sizeof(ra), (int)(((long long)e.Z * w.ld + mk::THREADS - 1) / mk::THREADS)));
+  }
+  CVG_TRY(fwd_generator(e, 2, true, true, label, d.B, d.Bg_bn, d.local_bn, st));
+  join_sides(e, st);
+  // the classifier branch (forward, loss, backward to x_fake) runs beside the critic's; they meet at ws.dx
+  const cudaStream_t sc = lambda_nonzero ? fork_to(e, 1, st) : st;
+  return score_fake(e, w.g_out + (size_t)e.F * w.ld, label, d, lambda_nonzero, st, sc);
+}
+
+// Seed and backward of ONE_CHAIN and THREE: once every side chain is done, both passes' seed, then the generator's and the
+// encoder's backward as one chain.
+static int eg_bwd_one(Engine& e, const SeedArgs& s, const BnNetBwd& gb, const BnNetBwd& eb, const StepDims& d,
+                      cudaStream_t st) {
+  join_sides(e, st);
+  CVG_TRY(launch_seed(e, s, 2, st));
+  CVG_TRY(bwd_bn_net(e, gb, d, st));
+  return bwd_bn_net(e, eb, d, st);
+}
+
+// Seed and backward of SPLIT: two chains, one per generator pass (their BatchNorm sums are per pass, and only pass 0 reaches
+// the encoder).
+//   caller's stream : seed and generator input gradients of pass 0, the encoder head gradient, the encoder backward
+//   side 1          : after the critic's and classifier's dx, seed and generator input gradients of pass 1
+//   side 0          : the generator's weight gradients, each after both passes' dY of its layer (one launch for both
+//                     passes, so the fixed-point sums are converted once, as with one chain)
+//   side 2          : the encoder's weight gradients, which must not queue behind the generator's
+static int eg_bwd_split(Engine& e, const SeedArgs& s, const BnNetBwd& gb, const BnNetBwd& eb, const StepDims& d,
+                        bool lambda_nonzero, cudaStream_t st) {
+  const cudaStream_t sA = e.ms.s[0], sB = e.ms.s[1];
+  CVG_TRY(launch_seed(e, s, 1, st));
+  SeedArgs s1 = s;                                   // pass 1 alone: dx through the sigmoid
+  s1.out += (size_t)e.F * e.ws.ld;
+  s1.dpre += (size_t)e.F * e.ws.ld;
+  s1.prior_only = 1;
+  if (lambda_nonzero) wait_for(e, sB, sA);           // the classifier's share of dx
+  CVG_TRY(launch_seed(e, s1, 1, sB));
+  for (int l = 3; l >= 0; --l) {
+    wait_for(e, sA, st);                             // dY of layer l, pass 0 ...
+    wait_for(e, sA, sB);                             // ... and pass 1
+    CVG_TRY(bwd_bn_dx(e, gb, l, d, st, 0));
+    if (l > 0) CVG_TRY(bwd_bn_dx(e, gb, l, d, sB, 1));
+    CVG_TRY(bwd_bn_dw(e, gb, l, d, sA));
+  }
+  for (int l = 3; l >= 0; --l) {
+    const cudaStream_t sw = fork_to(e, 2, st);       // dY of layer l
+    CVG_TRY(bwd_bn_dx(e, eb, l, d, st));
+    CVG_TRY(bwd_bn_dw(e, eb, l, d, sw));
+  }
+  return 0;
 }
 
 int step_g(Engine& e, const float* x_real, int label, int B, const CvgNoise* nz, const StepRng& rng, int flags,
@@ -1606,10 +1737,7 @@ int step_g(Engine& e, const float* x_real, int label, int B, const CvgNoise* nz,
   ProgramScope prog(e);
   CVG_TRY(begin_step(e, rng, true, st));
   const Workspace& w = e.ws;
-  const size_t ld = w.ld;
-  const bool local_bn = flags & CVG_STEP_LOCAL_BN;
-  const float Bg = (float)B * (float)e.world;
-  const float Bg_bn = local_bn ? (float)B : Bg;
+  const StepDims d = step_dims(e, B, flags);
   const int E = CVG_NET_ENCODER, G = CVG_NET_GENERATOR;
   if (rng.set) CVG_PAR(e);
   CVG_TRY(emit_zero(e, w.acc, w.acc_bytes, st));
@@ -1620,157 +1748,23 @@ int step_g(Engine& e, const float* x_real, int label, int B, const CvgNoise* nz,
   FillArgs f;
   fill_args(e, f, rng, B);
   // eps: slot 0 of ws.z for the stand-alone kernels (reparameterisation fused into the operand load); the program
-  // kernel keeps eps apart and materialises z_enc into slot 0 (mk::K_REPARAM below)
+  // kernel keeps eps apart and materialises z_enc into slot 0 (mk::K_REPARAM in eg_fwd_one)
   add_job(f, e.mk.recording ? w.z_eps : w.z, nz ? nz->eps : nullptr, 0, e.Z, 1, RS_EPS);
-  add_job(f, w.z + (size_t)e.Z * ld, nz ? nz->z : nullptr, 0, e.Z, 1, RS_Z);      // slot 1: z_prior
-  add_job(f, w.d_m1, nz ? nz->d_mask1 : nullptr, 1, e.dh[0], 1, RS_DMASK1);
-  add_job(f, w.d_m2, nz ? nz->d_mask2 : nullptr, 1, e.dh[1], 1, RS_DMASK2);
-  add_job(f, w.c_m1, nz ? nz->c_mask1 : nullptr, 1, e.ch[0], 1, RS_CMASK1);
-  add_job(f, w.c_m2, nz ? nz->c_mask2 : nullptr, 1, e.ch[1], 1, RS_CMASK2);
+  add_job(f, w.z + (size_t)e.Z * w.ld, nz ? nz->z : nullptr, 0, e.Z, 1, RS_Z);      // slot 1: z_prior
+  add_masks(e, f, CVG_NET_DISCRIMINATOR, nz, 1);
+  add_masks(e, f, CVG_NET_CLASSIFIER, nz, 1);
   CVG_PAR(e);
   CVG_TRY(launch_fill(e, f, st));
-  const float* x_fake = w.g_out + (size_t)e.F * ld;
-  CeArgs c;
-  c.M = B; c.ld = w.ld; c.K = e.K; c.npass = 1; c.label = label;
-  c.logits = w.c_logit; c.sl = (long long)e.K * ld;
-  c.dlogits = w.c_dlogit; c.sd = (long long)e.K * ld;
-  c.coef = 1.0f / Bg;       // times ctl->lambda_class, read on the device
-  c.ctl = w.ctl;
-  c.loss = w.loss + L_CE0;
-  // backward to x_fake: adv = -mean D(x_fake) (cvae_gan.py:189), then the classification term
-  const float seedv[2] = {-e.cfg.lambda_adv / Bg, 0.f};
-  // Three chains side by side (stand-alone kernels, side streams on; data parallel: with the folded exchange, one channel
-  // per chain): x_fake = G(z_prior) does not depend on the encoder, and the critic / classifier terms only on x_fake.
-  //   caller's stream : E(x), G(z_enc)
-  //   side 1          : batch staging, G(z_prior), then D(x_fake) forward and backward to x_fake
-  //   side 0          : power iteration, then C(x_fake) forward, loss and backward to x_fake (after D's: both add to ws.dx)
-  const bool three = !e.mk.recording && e.ms.on && (e.world <= 1 || local_bn || fold_stats(e, local_bn));
-  // The backward continues as two chains, one per generator pass (their BatchNorm sums are per pass, and only pass 0
-  // reaches the encoder):
-  //   caller's stream : seed and generator input gradients of pass 0, the encoder head gradient, the encoder backward
-  //   side 1          : after the critic's and classifier's dx, seed and generator input gradients of pass 1
-  //   side 0          : the generator's weight gradients, each after both passes' dY of its layer (one launch for both
-  //                     passes, so the fixed-point sums are converted once, as with one chain)
-  //   side 2          : the encoder's weight gradients, which must not queue behind the generator's
-  // Only where no BatchNorm sums are exchanged: a folded exchange of one pass cannot yet be told from the other pass's.
-  const bool split = three && e.eg_split && (e.world <= 1 || local_bn);
   join_sides(e, st);      // the previous step's Adam (visit: side stream 0) beside the fill just launched
-  if (three) {
-    const cudaStream_t sA = fork_to(e, 0, st), sB = fork_to(e, 1, st);
-    CVG_TRY(launch_sn(e, 1, true, sA));
-    CVG_TRY(stage_x(e, x_real, B, sB));
-    wait_for(e, st, sB);                                            // the encoder reads the staged batch
-    GenSplit prior;
-    prior.only_pass = 1; prior.channel = 1; prior.rec = e.ms.layer;
-    CVG_TRY(fwd_generator(e, 2, true, false, label, B, Bg_bn, local_bn, sB, nullptr, &prior));
-    wait_for(e, sB, sA);                                            // sigma of the critic's layers (all side 0 holds so far)
-    if (rng.lambda_nonzero) {
-      wait_for(e, sA, sB);                                          // x_fake
-      CVG_TRY(fwd_classifier(e, x_fake, 0, 1, true, B, sA));
-      CVG_TRY(emit_ce(e, c, B, 1, sA));
-    }
-    CVG_TRY(fwd_critic(e, x_fake, 0, 1, label, B, w.loss + L_DFAKE, sB));
-    CVG_TRY(bwd_critic(e, x_fake, 0, 1, label, B, seedv, false, true, sB));
-    if (rng.lambda_nonzero) CVG_TRY(bwd_classifier(e, x_fake, 0, 1, B, false, true, true, sA, sB));
-    CVG_TRY(fwd_encoder(e, true, label, B, Bg_bn, local_bn, st));
-    GenSplit enc;
-    enc.only_pass = 0; enc.channel = 0; enc.wait = e.ms.layer;
-    CVG_TRY(fwd_generator(e, 2, true, true, label, B, Bg_bn, local_bn, st, nullptr, &enc));
-    if (!split) join_sides(e, st);
-  } else {
-  CVG_PAR(e);
-  CVG_TRY(stage_x(e, x_real, B, fork_to(e, 1, st)));
-
-  CVG_PAR(e);
-  CVG_TRY(launch_sn(e, 1, true, fork_to(e, 0, st)));   // critic power iteration: independent of everything before D(x_fake)
-  // forward: E -> (mu, logvar); G on z_enc (pass 0) and z_prior (pass 1); D and C on x_fake
-  join_sides(e, st, 1);
-  CVG_TRY(fwd_encoder(e, true, label, B, Bg_bn, local_bn, st));
-  if (e.mk.recording) {
-    mk::ReparamArgs ra;
-    ra.mu = w.e_ml; ra.lv = w.e_ml + (size_t)e.Z * ld; ra.eps = w.z_eps; ra.out = w.z; ra.M = B; ra.ld = w.ld; ra.Z = e.Z;
-    CVG_TRY(mk_push(e, mk::K_REPARAM, &ra, sizeof(ra), (int)(((long long)e.Z * ld + mk::THREADS - 1) / mk::THREADS)));
-  }
-  CVG_TRY(fwd_generator(e, 2, true, true, label, B, Bg_bn, local_bn, st));
-  join_sides(e, st);
-  // the classifier branch (forward, loss, backward to x_fake) runs beside the critic's; they meet at ws.dx
-  const cudaStream_t sc = rng.lambda_nonzero ? fork_to(e, 1, st) : st;
-  CVG_TRY(fwd_critic(e, x_fake, 0, 1, label, B, w.loss + L_DFAKE, st));
-  CVG_TRY(fwd_classifier(e, x_fake, 0, 1, true, B, sc));
-  CVG_TRY(emit_ce(e, c, B, 1, sc));
-  CVG_TRY(bwd_critic(e, x_fake, 0, 1, label, B, seedv, false, true, st));
-  if (rng.lambda_nonzero) CVG_TRY(bwd_classifier(e, x_fake, 0, 1, B, false, true, true, sc, st));
-  join_sides(e, st);
-  }
-
+  const EgSchedule sched = eg_schedule(e, d.local_bn);
+  if (sched == EgSchedule::ONE_CHAIN) CVG_TRY(eg_fwd_one(e, x_real, label, d, rng.lambda_nonzero, st));
+  else CVG_TRY(eg_fwd_three(e, x_real, label, d, rng.lambda_nonzero, st));
   // generator output gradients: recon MSE on pass 0, dx on pass 1, through the sigmoid
-  SeedArgs s;
-  s.M = B; s.ld = w.ld; s.F = e.F;
-  s.out = w.g_out; s.sout = (long long)e.F * ld;
-  s.x = w.xT; s.dx = w.dx;
-  s.dpre = w.g_dout; s.sdpre = (long long)e.F * ld;
-  s.coef_recon = e.cfg.lambda_recon / (Bg * (float)e.F);
-  s.recon_acc = w.loss + L_RECON;
-  const unsigned seed_blocks = (unsigned)((e.F * ld + 255) / 256);
-  if (e.mk.recording) {
-    CVG_TRY(mk_push(e, mk::K_SEED, &s, sizeof(s), 2 * (int)(((long long)e.F * ld + mk::THREADS - 1) / mk::THREADS)));
-  } else if (split) {
-    const cudaStream_t sB = e.ms.s[1];
-    g_seed_kernel<<<dim3(seed_blocks, 1), 256, 0, st>>>(s);
-    CVG_LAUNCH_CHECK();
-    SeedArgs s1 = s;                                   // pass 1 alone: dx through the sigmoid
-    s1.out += (size_t)e.F * ld;
-    s1.dpre += (size_t)e.F * ld;
-    s1.prior_only = 1;
-    if (rng.lambda_nonzero) wait_for(e, sB, e.ms.s[0]);   // the classifier's share of dx
-    g_seed_kernel<<<dim3(seed_blocks, 1), 256, 0, sB>>>(s1);
-    CVG_LAUNCH_CHECK();
-  } else {
-    g_seed_kernel<<<dim3(seed_blocks, 2), 256, 0, st>>>(s);
-    CVG_LAUNCH_CHECK();
-  }
-
-  BnNetBwd gb;
-  gb.net = G; gb.npass = 2;
-  gb.h = w.g_h; gb.dy = w.g_dy;
-  gb.top_dy = w.g_dout; gb.s_top = (long long)e.F * ld;
-  gb.first_in.kind = e.mk.recording ? OP_PLAIN : OP_REPARAM; gb.first_in.rows = e.Z;
-  gb.first_in.p = w.z; gb.first_in.sp = (long long)e.Z * ld;
-  gb.first_in.mu = w.e_ml; gb.first_in.lv = w.e_ml + (size_t)e.Z * ld; gb.first_in.eps = w.z;
-  gb.first_in.reparam_pass = 0;
-  gb.first_K = e.Z;
-  gb.label_col = label_col_index(e, e.Z, label);
-  gb.want_first_dx = true;
-  const float kl_coef = e.cfg.lambda_kl / Bg;
-
-  BnNetBwd eb;
-  eb.net = E; eb.npass = 1;
-  eb.h = w.e_h; eb.dy = w.e_dy;
-  eb.top_dy = w.e_dml; eb.s_top = 0;
-  eb.first_in.kind = OP_PLAIN; eb.first_in.rows = e.F; eb.first_in.p = w.xT;
-  eb.first_K = e.F;
-  eb.label_col = label_col_index(e, e.F, label);
-  eb.want_first_dx = false;
-
-  if (split) {
-    const cudaStream_t sA = e.ms.s[0], sB = e.ms.s[1];
-    for (int l = 3; l >= 0; --l) {
-      wait_for(e, sA, st);                             // dY of layer l, pass 0 ...
-      wait_for(e, sA, sB);                             // ... and pass 1
-      CVG_TRY(bwd_bn_dx(e, gb, l, B, Bg_bn, kl_coef, local_bn, st, 0));
-      if (l > 0) CVG_TRY(bwd_bn_dx(e, gb, l, B, Bg_bn, kl_coef, local_bn, sB, 1));
-      CVG_TRY(bwd_bn_dw(e, gb, l, B, Bg_bn, local_bn, sA));
-    }
-    for (int l = 3; l >= 0; --l) {
-      const cudaStream_t sw = fork_to(e, 2, st);       // dY of layer l
-      CVG_TRY(bwd_bn_dx(e, eb, l, B, Bg_bn, 0.f, local_bn, st));
-      CVG_TRY(bwd_bn_dw(e, eb, l, B, Bg_bn, local_bn, sw));
-    }
-  } else {
-    CVG_TRY(bwd_bn_net(e, gb, B, Bg_bn, kl_coef, local_bn, st));
-    CVG_TRY(bwd_bn_net(e, eb, B, Bg_bn, 0.f, local_bn, st));
-  }
-
+  const SeedArgs s = seed_args(e, B, e.cfg.lambda_recon / (d.Bg * (float)e.F));
+  const BnNetBwd gb = gen_bwd(e, d, 2, e.mk.recording ? OP_PLAIN : OP_REPARAM, label, true);
+  const BnNetBwd eb = enc_bwd(e, label);
+  if (sched == EgSchedule::SPLIT) CVG_TRY(eg_bwd_split(e, s, gb, eb, d, rng.lambda_nonzero, st));
+  else CVG_TRY(eg_bwd_one(e, s, gb, eb, d, st));
   CVG_TRY(finish_step(e, (1 << E) | (1 << G), 2, B, flags, loss_out, st));
   return prog.finish(st);
 }
@@ -1790,8 +1784,7 @@ int step_g(Engine& e, const float* x_real, int label, int B, const CvgNoise* nz,
 // ------------------------------------------------------------------------------------------------
 static int hoist_generator(Engine& e, int nh, int label, int B, int flags, cudaStream_t st) {
   const Workspace& w = e.ws;
-  const bool local_bn = flags & CVG_STEP_LOCAL_BN;
-  const float Bg_bn = local_bn ? (float)B : (float)B * (float)e.world;
+  const StepDims d = step_dims(e, B, flags);
   StepRng rng;
   rng.set = false;
   rng.off = 1;
@@ -1808,7 +1801,7 @@ static int hoist_generator(Engine& e, int nh, int label, int B, int flags, cudaS
   GenBufs b;
   b.z = w.hz; b.out = w.hout;
   for (int l = 0; l < 3; ++l) { b.h[l] = w.hh[l]; b.fst[l] = w.hfst + (size_t)l * HOIST_MAX * 2 * STAT_C; }
-  return fwd_generator(e, nh, true, false, label, B, Bg_bn, local_bn, st, &b);
+  return fwd_generator(e, nh, true, false, label, B, d.Bg_bn, d.local_bn, st, &b);
 }
 
 int visit(Engine& e, int label, int B, int64_t B_global, const float* class_rows, int64_t n_rows, const float* x_batches,
