@@ -663,6 +663,7 @@ constexpr int DW_LDS = DW_MC + 4;  // padded row (conflict-free 128-bit reads ac
 // fixed point (DET_FIX_SCALE), where addition is exact and so independent of the order the CTAs finish in; the last CTA of
 // the tile (ticket on `tile_cnt`) converts the sums, adds them to the gradients and clears the slot and the counter.
 constexpr int DW_PART = 64 * 64 + 64;   // dW tile + bias sums
+constexpr int DW_FIN = 8;               // slot sums a finalising thread has in flight
 constexpr double DET_FIX_SCALE = 1099511627776.0;   // 2^40: resolution 9.1e-13, range +-8.4e6
 __device__ __forceinline__ unsigned long long det_fix(float v) {
   return (unsigned long long)__double2ll_rn((double)v * DET_FIX_SCALE);
@@ -804,17 +805,31 @@ __global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_dw_kernel(const DwArgs g
     unsigned long long* pa = tacc + (size_t)ps * DW_PART;
     float* dW = g.dW + (long long)ps * g.sdW;
     const bool bias = (g.db != nullptr || g.label_col >= 0) && blockIdx.x == 0;
-    for (int el = tid; el < DW_PART; el += GEMM_THREADS) {
-      const bool is_b = el >= 64 * 64;
-      const int n = n0 + (is_b ? el - 64 * 64 : el >> 6), k = k0 + (el & 63);
-      if (n >= g.N || (is_b ? !bias : k >= g.K)) continue;
-      const float sum = det_unfix(__ldcg(pa + el));
-      pa[el] = 0ull;
-      if (!is_b) {
-        atomicAdd(dW + (size_t)n * g.ldw + g.wcol0 + k, sum);
-      } else {
-        if (g.db) atomicAdd(g.db + n, sum);
-        if (g.label_col >= 0) atomicAdd(dW + (size_t)n * g.ldw + g.label_col, sum);
+    // This loop is the tail of every launch and runs in one CTA per tile.  Each thread reads DW_FIN sums before it writes
+    // any back, so their L2 round trips overlap instead of running one after another (the stores and atomics below
+    // may alias the slot as far as the compiler knows, so it cannot hoist the loads itself).
+    for (int base = tid; base < DW_PART; base += DW_FIN * GEMM_THREADS) {
+      unsigned long long v[DW_FIN];
+#pragma unroll
+      for (int u = 0; u < DW_FIN; ++u) {
+        const int el = base + u * GEMM_THREADS;
+        v[u] = el < DW_PART ? __ldcg(pa + el) : 0ull;
+      }
+#pragma unroll
+      for (int u = 0; u < DW_FIN; ++u) {
+        const int el = base + u * GEMM_THREADS;
+        if (el >= DW_PART) continue;
+        const bool is_b = el >= 64 * 64;
+        const int n = n0 + (is_b ? el - 64 * 64 : el >> 6), k = k0 + (el & 63);
+        if (n >= g.N || (is_b ? !bias : k >= g.K)) continue;
+        const float sum = det_unfix(v[u]);
+        pa[el] = 0ull;
+        if (!is_b) {
+          atomicAdd(dW + (size_t)n * g.ldw + g.wcol0 + k, sum);
+        } else {
+          if (g.db) atomicAdd(g.db + n, sum);
+          if (g.label_col >= 0) atomicAdd(dW + (size_t)n * g.ldw + g.label_col, sum);
+        }
       }
     }
   }
