@@ -670,23 +670,64 @@ __device__ __forceinline__ unsigned long long det_fix(float v) {
 }
 __device__ __forceinline__ float det_unfix(unsigned long long v) { return (float)((double)(long long)v / DET_FIX_SCALE); }
 
-template <int PK, int QK>
-__global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_dw_kernel(const DwArgs g, int nsplit, unsigned long long* acc64, unsigned* tile_cnt) {
+// The group launch (gemm_dw_group_kernel) has plain operands only (and the critic's constant seed), which need no transform
+// on their way to shared memory: it copies them there with cp.async, DW_STAGES - 1 chunks ahead of the FFMA block, so a CTA
+// keeps several chunks of L2 reads in flight without holding them in registers.  gemm_dw_kernel loads its operands to
+// registers one chunk ahead (load_raw / finish_operand), which every operand kind supports.
+constexpr int DW_STAGES = 4;
+// 16 bytes to shared memory, of which the first `bytes` from src and the rest zero
+__device__ __forceinline__ void cp_async16(float* dst, const float* src, int bytes) {
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;\n" ::"r"((unsigned)__cvta_generic_to_shared(dst)), "l"(src),
+               "r"(bytes));
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::); }
+template <int N>
+__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N)); }
+
+// A CTA's place in its weight-gradient launch: dW tile (kx, ny) of a launch kt tiles wide, pass-major batch slice z of the
+// launch's nz = g.npass x nsplit.  A launch of its own reads them from the grid at every use, as the kernel did before it
+// shared its body with the group: the compiler then sees that they are the same for the whole CTA, and compiles the
+// finalise's per-element branches without reconvergence points (with the values held in registers it did not, and the
+// widened model, whose weight gradients are all such launches, lost 1.8 % per visit).
+struct DwGridCta {
+  __device__ unsigned kx() const { return blockIdx.x; }
+  __device__ unsigned ny() const { return blockIdx.y; }
+  __device__ unsigned z() const { return blockIdx.z; }
+  __device__ unsigned kt() const { return gridDim.x; }
+  __device__ unsigned nz() const { return gridDim.z; }
+};
+// a member of a group launch (gemm_dw_group_kernel)
+struct DwMemberCta {
+  unsigned kx_, ny_, z_, kt_, nz_;
+  __device__ unsigned kx() const { return kx_; }
+  __device__ unsigned ny() const { return ny_; }
+  __device__ unsigned z() const { return z_; }
+  __device__ unsigned kt() const { return kt_; }
+  __device__ unsigned nz() const { return nz_; }
+};
+
+// One CTA of a weight-gradient launch at `cta`; acc64 / tile_cnt are the launch's fixed-point slots and ticket counters.
+// S: staged chunks (2: through registers; more: cp.async, plain operands only).  The staged values, and so every result,
+// are the same.
+template <int PK, int QK, int S, class Cta>
+__device__ __forceinline__ void dw_cta(const DwArgs& g, const Cta cta, int nsplit, unsigned long long* acc64,
+                                       unsigned* tile_cnt) {
+  static_assert(S == 2 || ((PK == OP_PLAIN || PK == OP_CONST) && QK == OP_PLAIN), "cp.async staging takes plain operands");
   extern __shared__ __align__(16) float dyn_smem[];
-  float* Ps = dyn_smem;                            // [2][64][DW_LDS]
-  float* Qs = Ps + 2 * 64 * DW_LDS;                // [2][64][DW_LDS]
-  float* cs_p = Qs + 2 * 64 * DW_LDS;
+  float* Ps = dyn_smem;                            // [S][64][DW_LDS]
+  float* Qs = Ps + S * 64 * DW_LDS;                // [S][64][DW_LDS]
+  float* cs_p = Qs + S * 64 * DW_LDS;
   float* cs_q = cs_p + operand_const_floats(g.p);
 
   const int tid = threadIdx.x;
-  const int pass = blockIdx.z / nsplit, split = blockIdx.z % nsplit;
-  const int k0 = blockIdx.x * 64, n0 = blockIdx.y * 64;
+  const int pass = cta.z() / nsplit, split = cta.z() % nsplit;
+  const int k0 = cta.kx() * 64, n0 = cta.ny() * 64;
   const int mbeg = split * g.rows_per_cta;
   const int mend = min(g.M, mbeg + g.rows_per_cta);
 
   const NvlDev* poll_p = ((PK == OP_BN_ACT || PK == OP_BN_BWD) && g.p.bn.poll) ? g.nvl : nullptr;
   const NvlDev* poll_q = ((QK == OP_BN_ACT || QK == OP_BN_BWD) && g.q.bn.poll) ? g.nvl : nullptr;
-  if ((poll_p || poll_q) && blockIdx.x == 0 && blockIdx.y == 0 && split == 0) {   // this pass's write-back CTA
+  if ((poll_p || poll_q) && cta.kx() == 0 && cta.ny() == 0 && split == 0) {   // this pass's write-back CTA
     if (poll_p) { bn_poll_writeback(g.p.bn, pass, 1, poll_p); if (g.p.bn.poll >> 20) bn_publish(g.p.bn, pass, 1); }
     if (poll_q) { bn_poll_writeback(g.q.bn, pass, 1, poll_q); if (g.q.bn.poll >> 20) bn_publish(g.q.bn, pass, 1); }
     __syncthreads();
@@ -710,7 +751,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_dw_kernel(const DwArgs g
 #pragma unroll
     for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
   float bsum[4] = {0.f, 0.f, 0.f, 0.f};
-  const bool do_bias = (g.db != nullptr || g.label_col >= 0) && blockIdx.x == 0 && tk == 0;
+  const bool do_bias = (g.db != nullptr || g.label_col >= 0) && cta.kx() == 0 && tk == 0;
 
   struct Regs { Raw p[2], q[2]; };
   auto gload = [&](int mb, Regs& r) {
@@ -759,21 +800,50 @@ __global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_dw_kernel(const DwArgs g
   };
 
   const int nchunks = mbeg < mend ? (mend - mbeg + DW_MC - 1) / DW_MC : 0;
-  Regs rr;
-  if (nchunks > 0) {
-    gload(mbeg, rr);
-    sstore(0, mbeg, rr);
-  }
-  __syncthreads();
-  for (int c = 0; c < nchunks; ++c) {
-    const int cur = c & 1;
-    if (c + 1 < nchunks) gload(mbeg + (c + 1) * DW_MC, rr);
-    compute(cur);
-    if (c + 1 < nchunks) sstore(cur ^ 1, mbeg + (c + 1) * DW_MC, rr);
+  if constexpr (S > 2) {
+    // the same values finish_operand<OP_PLAIN> gives: rows >= mend and feature rows >= o.rows are zero-filled
+    auto copy_plain = [&](const Operand& o, float* dst, int r, int m) {
+      const int bytes = (r < o.rows && m < mend) ? 4 * min(4, mend - m) : 0;
+      cp_async16(dst, bytes ? o.p + (long long)pass * o.sp + (size_t)r * g.ld + m : o.p, bytes);
+    };
+    auto stage = [&](int buf, int mb) {   // one commit group per chunk
+#pragma unroll
+      for (int t = 0; t < 2; ++t) {
+        const int row = l_row + 32 * t;
+        float* dp = Ps + ((size_t)buf * 64 + row) * DW_LDS + l_m;
+        if (PK == OP_PLAIN) copy_plain(g.p, dp, n0 + row, mb + l_m);
+        else st4(dp, finish_operand<PK>(g.p, cs_p, pass, n0 + row, mb + l_m, mend, g.slope, Raw{}));
+        copy_plain(g.q, Qs + ((size_t)buf * 64 + row) * DW_LDS + l_m, k0 + row, mb + l_m);
+      }
+    };
+    for (int c = 0; c < S - 1; ++c) {
+      if (c < nchunks) stage(c, mbeg + c * DW_MC);
+      cp_async_commit();
+    }
+    for (int c = 0; c < nchunks; ++c) {
+      cp_async_wait<S - 2>();   // this thread's copies of chunk c have landed ...
+      __syncthreads();          // ... and everyone's; every thread is done with chunk c - 1, whose buffer is refilled now
+      if (c + S - 1 < nchunks) stage((c + S - 1) % S, mbeg + (c + S - 1) * DW_MC);
+      cp_async_commit();
+      compute(c % S);
+    }
+  } else {
+    Regs rr;
+    if (nchunks > 0) {
+      gload(mbeg, rr);
+      sstore(0, mbeg, rr);
+    }
     __syncthreads();
+    for (int c = 0; c < nchunks; ++c) {
+      const int cur = c & 1;
+      if (c + 1 < nchunks) gload(mbeg + (c + 1) * DW_MC, rr);
+      compute(cur);
+      if (c + 1 < nchunks) sstore(cur ^ 1, mbeg + (c + 1) * DW_MC, rr);
+      __syncthreads();
+    }
   }
 
-  const int tile = blockIdx.y * gridDim.x + blockIdx.x;
+  const int tile = cta.ny() * cta.kt() + cta.kx();
   unsigned long long* tacc = acc64 + (size_t)tile * g.npass * DW_PART;
   {
     unsigned long long* mine = tacc + (size_t)pass * DW_PART;
@@ -790,7 +860,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_dw_kernel(const DwArgs g
   __threadfence();
   __syncthreads();
   __shared__ unsigned s_last;
-  if (tid == 0) s_last = atomicAdd(tile_cnt + tile, 1u) == gridDim.z - 1 ? 1u : 0u;
+  if (tid == 0) s_last = atomicAdd(tile_cnt + tile, 1u) == cta.nz() - 1 ? 1u : 0u;
   __syncthreads();
   if (!s_last) return;
   __threadfence();
@@ -804,7 +874,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_dw_kernel(const DwArgs g
     }
     unsigned long long* pa = tacc + (size_t)ps * DW_PART;
     float* dW = g.dW + (long long)ps * g.sdW;
-    const bool bias = (g.db != nullptr || g.label_col >= 0) && blockIdx.x == 0;
+    const bool bias = (g.db != nullptr || g.label_col >= 0) && cta.kx() == 0;
     // This loop is the tail of every launch and runs in one CTA per tile.  Each thread reads DW_FIN sums before it writes
     // any back, so their L2 round trips overlap instead of running one after another (the stores and atomics below
     // may alias the slot as far as the compiler knows, so it cannot hoist the loads itself).
@@ -836,6 +906,42 @@ __global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_dw_kernel(const DwArgs g
   if (tid == 0) tile_cnt[tile] = 0u;
 }
 
+template <int PK, int QK>
+__global__ void __launch_bounds__(GEMM_THREADS, 2)
+    gemm_dw_kernel(const __grid_constant__ DwArgs g, int nsplit, unsigned long long* acc64, unsigned* tile_cnt) {
+  dw_cta<PK, QK, 2>(g, DwGridCta{}, nsplit, acc64, tile_cnt);
+}
+
+// Several independent weight gradients in one launch (the four layers of a D or C step after its fused chain).  Each
+// member is the launch gemm_dw_kernel would make of it: its CTAs, in the same order, occupy [first, first + its CTA count)
+// of a flat grid, with its own slots and counters at acc_off / cnt_off of the stream's set.
+constexpr int DW_GROUP_MAX = 5;
+struct DwMember {
+  DwArgs g;                        // g.p: OP_PLAIN or OP_CONST, g.q: OP_PLAIN
+  int nsplit = 1, kt = 1, nt = 1;
+  int first = 0;
+  long long acc_off = 0;
+  int cnt_off = 0;
+};
+struct DwGroup {
+  DwMember m[DW_GROUP_MAX];
+  int n = 0;
+};
+
+__global__ void __launch_bounds__(GEMM_THREADS, 2)
+    gemm_dw_group_kernel(const __grid_constant__ DwGroup grp, unsigned long long* acc64, unsigned* tile_cnt) {
+  int i = 0;
+  while (i + 1 < grp.n && (int)blockIdx.x >= grp.m[i + 1].first) ++i;
+  const DwMember& mb = grp.m[i];
+  const int local = (int)blockIdx.x - mb.first, tiles = mb.kt * mb.nt;
+  const DwMemberCta cta{(unsigned)(local % mb.kt), (unsigned)((local % tiles) / mb.kt), (unsigned)(local / tiles), (unsigned)mb.kt,
+                        (unsigned)(mb.g.npass * mb.nsplit)};
+  if (mb.g.p.kind == OP_CONST)
+    dw_cta<OP_CONST, OP_PLAIN, DW_STAGES>(mb.g, cta, mb.nsplit, acc64 + mb.acc_off, tile_cnt + mb.cnt_off);
+  else
+    dw_cta<OP_PLAIN, OP_PLAIN, DW_STAGES>(mb.g, cta, mb.nsplit, acc64 + mb.acc_off, tile_cnt + mb.cnt_off);
+}
+
 inline size_t gemm_mn_smem(const GemmArgs& g) {
   size_t f = operand_const_floats(g.a);
   if (g.ekind == EP_DBN) f += 4 * (size_t)g.prev_bn.C;
@@ -843,8 +949,8 @@ inline size_t gemm_mn_smem(const GemmArgs& g) {
   f += 4 * (size_t)TBN * RED_LD;   // split-K partial tiles
   return f * sizeof(float);
 }
-inline size_t gemm_dw_smem(const DwArgs& g) {
-  size_t f = 4 * 64 * DW_LDS + operand_const_floats(g.p) + operand_const_floats(g.q);
+inline size_t gemm_dw_smem(const DwArgs& g, int stages = 2) {
+  size_t f = 2 * (size_t)stages * 64 * DW_LDS + operand_const_floats(g.p) + operand_const_floats(g.q);
   return f * sizeof(float);
 }
 

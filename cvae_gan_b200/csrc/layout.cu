@@ -1,4 +1,5 @@
 // cvaegan_b200 - network layouts (reference state_dict keys -> offsets) and workspace carving.
+#include <algorithm>
 #include "engine.cuh"
 
 namespace cvg {
@@ -257,8 +258,21 @@ static size_t carve(const Engine& e, Workspace& w, void* base) {
         tiles = std::max(tiles, ((p.in + 63) / 64) * ((p.out + 63) / 64));
         cmax = std::max(cmax, std::max(p.in, p.out));
       }
-    w.det_acc_n = std::max((long long)tiles * DET_MAX_PASS * DW_PART, 2LL * cmax);
-    w.det_cnt_n = tiles;
+    // the D and C steps' weight gradients after their chains: one group launch (launch_dw_group) of every layer, two passes
+    // each, its members' tiles side by side; the critic's last layer runs as two one-pass members with a counter each.
+    // An upper bound: it counts the critic's first layer with its label columns (the group's member has F), and models
+    // whose widths the chains do not take never launch a group.  launch_dw_group checks the actual group against it.
+    int group_tiles = 0;
+    for (int net : {CVG_NET_DISCRIMINATOR, CVG_NET_CLASSIFIER}) {
+      int t = 0;
+      for (int i = 0; i < e.lay[net].nlin; ++i) {
+        const LinearP& p = e.lay[net].lin[i];
+        t += ((p.in + 63) / 64) * ((p.out + 63) / 64) * (net == CVG_NET_DISCRIMINATOR && i == e.lay[net].nlin - 1 ? 2 : 1);
+      }
+      group_tiles = std::max(group_tiles, t);
+    }
+    w.det_acc_n = std::max({(long long)tiles * DET_MAX_PASS * DW_PART, (long long)group_tiles * 2 * DW_PART, 2LL * cmax});
+    w.det_cnt_n = std::max(tiles, group_tiles);
     for (int i = 0; i < SIDE_STREAMS + 1; ++i) {
       w.det_acc[i] = c.take<unsigned long long>((size_t)w.det_acc_n);
       w.det_cnt[i] = c.take<unsigned>((size_t)w.det_cnt_n);

@@ -1,6 +1,7 @@
 // cvaegan_b200 - the three optimiser steps of a label visit (cvae_gan.py:104-216), as sequences of
 // fused kernels on one stream.  Data parallel: batch rows are sharded; BatchNorm batch moments and
 // the flat gradient buffers are all-reduced with NCCL between / after the kernels.
+#include <algorithm>
 #include <dlfcn.h>
 #include <math.h>
 
@@ -272,19 +273,28 @@ static int det_slot(const Engine& e, cudaStream_t st) {
   return 0;
 }
 
-int launch_dw(Engine& e, const DwArgs& g0, cudaStream_t st) {
-  if (e.mk.recording) return mk_push_dw(e, g0);
-  DwArgs g = g0;
-  const int kt = (g.K + 63) / 64, nt = (g.N + 63) / 64;
+// Split-batch partition of a weight gradient: kt x nt tiles of 64 x 64, each pass's batch split into nsplit slices of
+// g.rows_per_cta rows (a multiple of DW_MC), about two CTAs per SM in all.  It fixes the fixed-point partials, and so the
+// last bits of the gradient: every launch of a given weight gradient must split it the same way.
+static int dw_split(const Engine& e, DwArgs& g, int* kt, int* nt) {
+  *kt = (g.K + 63) / 64;
+  *nt = (g.N + 63) / 64;
   const int target = 2 * e.num_sms;
-  int nsplit = (target + kt * nt * g.npass - 1) / (kt * nt * g.npass);
+  int nsplit = (target + *kt * *nt * g.npass - 1) / (*kt * *nt * g.npass);
   const int max_split = (g.M + DW_MC - 1) / DW_MC;
   if (nsplit > max_split) nsplit = max_split;
   if (nsplit < 1) nsplit = 1;
   int rows = (g.M + nsplit - 1) / nsplit;
   rows = ((rows + DW_MC - 1) / DW_MC) * DW_MC;
-  nsplit = (g.M + rows - 1) / rows;
   g.rows_per_cta = rows;
+  return (g.M + rows - 1) / rows;
+}
+
+int launch_dw(Engine& e, const DwArgs& g0, cudaStream_t st) {
+  if (e.mk.recording) return mk_push_dw(e, g0);
+  DwArgs g = g0;
+  int kt, nt;
+  const int nsplit = dw_split(e, g, &kt, &nt);
   if (const NvlDev* ch = take_pending(e, g.p)) g.nvl = ch;
   if (const NvlDev* ch = take_pending(e, g.q)) g.nvl = ch;
   dim3 grid(kt, nt, g.npass * nsplit);
@@ -297,6 +307,47 @@ int launch_dw(Engine& e, const DwArgs& g0, cudaStream_t st) {
   if (err != cudaSuccess)
     CVG_FAIL(std::string("gemm_dw launch (p.kind ") + std::to_string(g.p.kind) + ", q.kind " + std::to_string(g.q.kind) +
              "): " + cudaGetErrorString(err));
+  e.launches++;
+  return 0;
+}
+
+// Independent weight gradients as one launch (gemm_dw_group_kernel), each partitioned and reduced exactly as launch_dw
+// would.  Members with more batch chunks per CTA come first in the grid, so their long CTAs are dispatched first.  Only
+// plain operands (and the critic's constant seed): no BatchNorm constants, no exchanges in flight.
+static int launch_dw_group(Engine& e, const DwArgs* members, int n, cudaStream_t st) {
+  if (n < 1 || n > DW_GROUP_MAX) CVG_FAIL("internal: weight-gradient group of " + std::to_string(n) + " members");
+  DwGroup grp;
+  grp.n = n;
+  for (int i = 0; i < n; ++i) {
+    DwMember& m = grp.m[i];
+    m.g = members[i];
+    if ((m.g.p.kind != OP_PLAIN && m.g.p.kind != OP_CONST) || m.g.q.kind != OP_PLAIN || m.g.p.bn.poll || m.g.q.bn.poll ||
+        m.g.nvl)
+      CVG_FAIL("internal: weight-gradient group member with BatchNorm operands or an exchange");
+    m.nsplit = dw_split(e, m.g, &m.kt, &m.nt);
+  }
+  std::stable_sort(grp.m, grp.m + n, [](const DwMember& a, const DwMember& b) { return a.g.rows_per_cta > b.g.rows_per_cta; });
+  long long acc = 0;
+  int cnt = 0, ctas = 0;
+  double flops = 0.0;
+  for (int i = 0; i < n; ++i) {
+    DwMember& m = grp.m[i];
+    m.first = ctas;
+    m.acc_off = acc;
+    m.cnt_off = cnt;
+    ctas += m.kt * m.nt * m.g.npass * m.nsplit;
+    acc += (long long)m.kt * m.nt * m.g.npass * DW_PART;
+    cnt += m.kt * m.nt;
+    flops += 2.0 * m.g.M * (double)m.g.N * m.g.K * m.g.npass;
+  }
+  if (acc > e.ws.det_acc_n || cnt > e.ws.det_cnt_n)
+    CVG_FAIL("internal: weight-gradient group exceeds the deterministic-reduction slots");
+  const int slot = det_slot(e, st);
+  prof_begin(e, 2, flops, st);
+  gemm_dw_group_kernel<<<ctas, GEMM_THREADS, gemm_dw_smem(grp.m[0].g, DW_STAGES), st>>>(grp, e.ws.det_acc[slot], e.ws.det_cnt[slot]);
+  const cudaError_t err = cudaGetLastError();
+  prof_end(e, st);
+  if (err != cudaSuccess) CVG_FAIL(std::string("gemm_dw_group launch: ") + cudaGetErrorString(err));
   e.launches++;
   return 0;
 }
@@ -734,10 +785,6 @@ static bool chain_usable(const Engine& e, int net) {
   return h[0] == CH_H0 && h[1] == CH_H1 && h[2] == CH_H2 && e.F <= CH_MAX_IN && e.K <= CH_MAX_K;
 }
 
-// After a chain the weight gradients of the four layers are independent of each other: the largest (layer 1) runs on the
-// caller's stream, the others beside it on the side streams (each stream has its own deterministic-reduction slot).
-static cudaStream_t chain_dw_stream(Engine& e, int l, cudaStream_t st) { return l == 1 ? st : fork_to(e, l == 2 ? 1 : 0, st); }
-
 // Critic forward (score sums into loss[L_DREAL + pass]) and input gradients from the per-pass seed, both passes, one launch.
 static int launch_critic_chain(Engine& e, long long sx, int label, int M, const float* seed, cudaStream_t st) {
   const int net = CVG_NET_DISCRIMINATOR;
@@ -809,8 +856,8 @@ static int launch_classifier_chain(Engine& e, long long sx, int label, int M, fl
 // ------------------------------------------------------------------------------------------------
 // critic backward.  seed[pass] = dL/dscore (constant over rows).  want_dw: accumulate per-pass raw
 // gradients into ws.sn_G (+ bias grads into the grad buffer).  want_dx: write dL/dx into ws.dx.
-// dw_only: a fused chain (chain.cuh) has produced the input gradients; only the weight gradients are launched, spread over
-// the streams (chain_dw_stream).
+// dw_only: a fused chain (chain.cuh) has produced the input gradients; the weight gradients, independent of each other
+// now, run as one group launch on st (launch_dw_group).
 static int bwd_critic(Engine& e, const float* xin, long long sxin, int npass, int label, int M, const float* seed,
                       bool want_dw, bool want_dx, cudaStream_t st, bool dw_only = false) {
   const int net = CVG_NET_DISCRIMINATOR;
@@ -818,6 +865,8 @@ static int bwd_critic(Engine& e, const float* xin, long long sxin, int npass, in
   const size_t ld = w.ld;
   const float keep_inv = 1.0f / (1.0f - e.cfg.dropout_p);
   const long long sG = e.lay[net].n_param;
+  DwArgs group[DW_GROUP_MAX];
+  int ngroup = 0;
   for (int l = 3; l >= 0; --l) {
     const LinearP& p = lin(e, net, l);
     // dY operand of this layer
@@ -831,7 +880,7 @@ static int bwd_critic(Engine& e, const float* xin, long long sxin, int npass, in
       // OP_CONST carries one value: run the two passes of layer 4 as separate launches
       const int reps = (l == 3 && npass > 1) ? npass : 1;
       // beside the input-gradient chain: both only read dY of layer l
-      const cudaStream_t sw = dw_only ? chain_dw_stream(e, l, st) : fork_to(e, 0, st);
+      const cudaStream_t sw = dw_only ? st : fork_to(e, 0, st);
       for (int r = 0; r < reps; ++r) {
         if (r > 0) CVG_PAR(e);
         DwArgs d = base_dw(e, M, (float)M, reps > 1 ? 1 : npass);
@@ -848,7 +897,8 @@ static int bwd_critic(Engine& e, const float* xin, long long sxin, int npass, in
         d.ldw = p.in;
         d.db = (l == 3) ? nullptr : e.G(net, p.b);   // score-bias gradient is added analytically (sn_grad_kernel)
         d.label_col = (l == 0) ? label_col_index(e, e.F, label) : -1;
-        CVG_TRY(launch_dw(e, d, sw));
+        if (dw_only) group[ngroup++] = d;
+        else CVG_TRY(launch_dw(e, d, sw));
       }
     }
     if (dw_only) continue;
@@ -888,6 +938,7 @@ static int bwd_critic(Engine& e, const float* xin, long long sxin, int npass, in
       }
     }
   }
+  if (ngroup) return launch_dw_group(e, group, ngroup, st);
   return 0;
 }
 
@@ -900,6 +951,8 @@ static int bwd_classifier(Engine& e, const float* xin, long long sxin, int npass
   const Workspace& w = e.ws;
   const size_t ld = w.ld;
   const float keep_inv = 1.0f / (1.0f - e.cfg.dropout_p);
+  DwArgs group[DW_GROUP_MAX];
+  int ngroup = 0;
   for (int l = 3; l >= 0; --l) {
     const LinearP& p = lin(e, net, l);
     Operand dy;
@@ -922,7 +975,8 @@ static int bwd_classifier(Engine& e, const float* xin, long long sxin, int npass
       d.sdW = 0;
       d.ldw = p.in;
       d.db = e.G(net, p.b);
-      CVG_TRY(launch_dw(e, d, dw_only ? chain_dw_stream(e, l, st) : fork_to(e, 0, st)));
+      if (dw_only) group[ngroup++] = d;
+      else CVG_TRY(launch_dw(e, d, fork_to(e, 0, st)));
     }
     if (dw_only) continue;
     if (l == 0 && !want_dx) break;
@@ -971,6 +1025,8 @@ static int bwd_classifier(Engine& e, const float* xin, long long sxin, int npass
       }
     }
   }
+  // after the chain, whose LayerNorm affine sums use this stream's slot and counters too: both leave them cleared
+  if (ngroup) return launch_dw_group(e, group, ngroup, st);
   return 0;
 }
 
@@ -1871,6 +1927,7 @@ void set_all_kernel_attributes() {
   CVG_DW_ATTR(OP_PLAIN, OP_PLAIN) CVG_DW_ATTR(OP_CONST, OP_PLAIN) CVG_DW_ATTR(OP_PLAIN, OP_BN_ACT)
   CVG_DW_ATTR(OP_BN_BWD, OP_BN_ACT) CVG_DW_ATTR(OP_BN_BWD, OP_REPARAM) CVG_DW_ATTR(OP_BN_BWD, OP_PLAIN)
 #undef CVG_DW_ATTR
+  cudaFuncSetAttribute(gemm_dw_group_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
 }
 
 }  // namespace cvg
